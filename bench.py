@@ -4,6 +4,7 @@ at 2^24, on N B200s of one node, with the host-CPU restatement of the reference 
 
     python bench.py --gpus N --steps K --warmup W            # this repo (sm_100a CUDA path through the C ABI)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm (oracle port), host cores
+    python bench.py ... --dump-outputs DIR                   # + the outputs of every timed leg's last step, DIR/*.npy
 
 One JSON line on stdout.  Top-level value = MSM points/s (inputs resident in HBM); `sumcheck` holds the second half of
 the metric; `e2e` = the same MSM through the public API from pinned HOST buffers (H2D + D2H inside the timed region).
@@ -15,6 +16,7 @@ Inputs (0.5 GiB scalars + 1 GiB bases; 1.5 GiB tables) are far larger than the 1
 from __future__ import annotations
 
 import argparse
+import dataclasses
 import json
 import os
 import subprocess
@@ -143,6 +145,32 @@ def product_expr(q, k):
     for i in range(1, k):
         e = e * q.VirtualPolyExpr.Input(i)
     return e
+
+
+def output_bytes(o) -> list:
+    """The byte arrays of one output (a G1 point, a transcript state, or a proof built of dataclasses, lists and tuples
+    of them) in field order; integer fields (num_vars) follow from the arguments and are left out."""
+    import numpy as np
+    if dataclasses.is_dataclass(o):
+        return [b for f in dataclasses.fields(o) for b in output_bytes(getattr(o, f.name))]
+    if isinstance(o, (list, tuple)):
+        return [b for x in o for b in output_bytes(x)]
+    if isinstance(o, bytes):
+        return [np.frombuffer(o, dtype=np.uint8)]
+    if isinstance(o, np.ndarray):
+        return [np.ascontiguousarray(o).view(np.uint8).reshape(-1)]
+    return []
+
+
+def dump_outputs(path: str, outputs: dict) -> None:
+    """--dump-outputs: each output as PATH/<name>.npy, the float64 vector of its little-endian 32-bit limbs (Montgomery
+    form for field elements and points, as the API returns them).  Every limb is below 2^53, so the values are exact and
+    two builds can be compared output for output.  The outputs are proofs and commitments: a few hundred KB at most."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, o in outputs.items():
+        b = np.concatenate([np.zeros(0, dtype=np.uint8)] + output_bytes(o))
+        np.save(os.path.join(path, name + ".npy"), b.view("<u4").astype(np.float64))
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -274,7 +302,7 @@ def imad_roofline(stats, imad_peak, step_ms, steps):
             "traffic": None, "peak_source": "qz_bench_imad measured in this run"}
 
 
-def bench_hyperplonk(ctx, q, log_rows, g_bytes, tau_mont, timed_loop, verify=False):
+def bench_hyperplonk(ctx, q, log_rows, g_bytes, tau_mont, timed_loop, steps, verify=False):
     """BASELINE.json config 5 shape: two traces (Fibonacci, 4 columns; modified Fibonacci, 5 columns padded to 8) of
     2^log_rows rows each, proved with HyperPlonk::prove (zero-check + logup permutation check + MLPCS openings)."""
     import numpy as np
@@ -344,7 +372,7 @@ def bench_hyperplonk(ctx, q, log_rows, g_bytes, tau_mont, timed_loop, verify=Fal
     out = {}
     out["p"] = prover.prove(kzg, witnesses)  # warm-up proof (untimed)
     ctx.msm_accumulate_stats(1)
-    ms, launches = timed_loop(lambda: out.__setitem__("p", prover.prove(kzg, witnesses)), 1, 0)
+    ms, launches = timed_loop(lambda: out.__setitem__("p", prover.prove(kzg, witnesses)), steps, 0)
     acc_stats = ctx.msm_accumulate_stats(-1)
     kzg.srs.free()
     verified = None
@@ -370,9 +398,9 @@ def bench_hyperplonk(ctx, q, log_rows, g_bytes, tau_mont, timed_loop, verify=Fal
     return {"value": ms * 1e-3, "unit": "s per proof", "rows_per_trace": rows, "traces": 2, "columns": [4, 8],
             "verified": verified, "verified_by": "oracle/verifier.py hyperplonk_verify (restated reference verifier incl. BN254 pairings), "
             f"{verify_s:.1f} s on the host after the timed region" if verify else None,
-            "gpu_launches": launches, "workload": "HyperPlonk::prove of Fibonacci + modified-Fibonacci transition circuits "
+            "gpu_launches": launches // steps, "workload": "HyperPlonk::prove of Fibonacci + modified-Fibonacci transition circuits "
             "(2 witness commits, 2 zero-checks, 2 logup permutation checks, 2 x (cols + public + 5) MLPCS openings)",
-            "final_transcript_state": out["p"].transcript_state.hex(), "_acc_stats": acc_stats, "_ms": ms}
+            "final_transcript_state": out["p"].transcript_state.hex(), "_acc_stats": acc_stats, "_ms": ms, "_proof": out["p"]}
 
 
 def run_gpu(args):
@@ -558,9 +586,9 @@ def run_gpu(args):
 
         commit_open()  # warm-up (untimed)
         ctx.msm_accumulate_stats(1)
-        ml_ms, ml_launches = timed_loop(commit_open, max(1, args.steps // 2), 0)
+        ml_ms, ml_launches = timed_loop(commit_open, args.steps, 0)
         ml_stats = ctx.msm_accumulate_stats(-1)
-        mlpcs = {"_acc_stats": ml_stats, "_ms": ml_ms, "_steps": max(1, args.steps // 2), "value": ml_ms * 1e-3, "unit": "s per commit+open", "log_n": nm, "gpu_launches": ml_launches // max(1, args.steps // 2),
+        mlpcs = {"_acc_stats": ml_stats, "_ms": ml_ms, "value": ml_ms * 1e-3, "unit": "s per commit+open", "log_n": nm, "gpu_launches": ml_launches // args.steps,
                  "workload": f"MultilinearPCS::commit + ::open of a 2^{nm}-entry MLE (6 MSMs, eq table, NTT 2^{nm + 1}, 4 quotients)"}
         poly.free()
 
@@ -569,7 +597,7 @@ def run_gpu(args):
     hplonk = None
     if args.hyperplonk_log_rows > 0:
         hplonk = bench_hyperplonk(ctx, q, args.hyperplonk_log_rows, np.concatenate([mont(1, FQ), mont(2, FQ)]), mont(TAU),
-                                  timed_loop, verify=rank == 0 and not args.no_verify)
+                                  timed_loop, args.steps, verify=rank == 0 and not args.no_verify)
         hplonk["n_gpus"] = world
 
 
@@ -653,14 +681,29 @@ def run_gpu(args):
         if pair_leg:
             line["msm_pair_levels"] = pair_leg
         if mlpcs:
-            mlpcs["roofline"] = imad_roofline(mlpcs.pop("_acc_stats"), imad_peak, mlpcs.pop("_ms"), mlpcs.pop("_steps"))
+            mlpcs["roofline"] = imad_roofline(mlpcs.pop("_acc_stats"), imad_peak, mlpcs.pop("_ms"), args.steps)
             line["mlpcs_commit_open"] = mlpcs
+        hp_proof = None
         if hplonk:
-            hplonk["roofline"] = imad_roofline(hplonk.pop("_acc_stats"), imad_peak, hplonk.pop("_ms"), 1)
+            hp_proof = hplonk.pop("_proof")
+            hplonk["roofline"] = imad_roofline(hplonk.pop("_acc_stats"), imad_peak, hplonk.pop("_ms"), args.steps)
             line["hyperplonk_prove"] = hplonk
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline(args)
         print(json.dumps(line))
+        if args.dump_outputs:
+            # what each timed leg returned to its caller in its last step
+            outputs = {"msm_commitment": results["dev"], "msm_commitment_host_scalars": results["host"],
+                       "msm_pair_levels_commitment": results.get("pair") if pair_leg and "error" not in pair_leg else None,
+                       "sumcheck_proof": sc_out["dev"], "sumcheck_transcript_state": sc_out["dev_state"],
+                       "sumcheck_proof_host_tables": sc_out["host"],
+                       "sumcheck_transcript_state_host_tables": sc_out["host_state"],
+                       "zerocheck_proof": sc_out.get("zc") if zc_err is None else None,
+                       "zerocheck_transcript_state": sc_out.get("zc_state") if zc_err is None else None,
+                       "msm_2_20_commitment": results.get("c20"),
+                       "mlpcs_commitment": results.get("ml_c"), "mlpcs_opening": results.get("ml_o"),
+                       "hyperplonk_proof": hp_proof}
+            dump_outputs(args.dump_outputs, {k: v for k, v in outputs.items() if v is not None})
     for b in tabs_dev + [scal_dev]:
         b.free()
     kzg.srs.free()
@@ -689,7 +732,14 @@ def main():
     ap.add_argument("--no-verify", action="store_true", help="skip the verifier check of the HyperPlonk proof")
     ap.add_argument("--no-precompute", action="store_true", help="MSM without the precomputed window multiples")
     ap.add_argument("--precompute-bits", type=int, default=0, help="window bits of the precomputed table (0 = auto)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what every timed leg returned in "
+                    "its last step as DIR/<name>.npy (float64 32-bit limbs; the inputs are seeded, so runs with the same "
+                    "arguments compare output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = max(args.warmup, 1)
     if args.impl == "reference":
