@@ -44,20 +44,33 @@ def gpu_prove(ctx, n, tables, nodes, consts, claimed, domain, zerocheck=False, d
     return sc, claim, tr.state.copy(), z
 
 
-def assert_same(ctx, n, tables, nodes, consts, claimed, domain, zerocheck=False, device_tables=False, threads=1):
-    sc, claim, state, z = gpu_prove(ctx, n, tables, nodes, consts, claimed, domain, zerocheck, device_tables)
+def oracle_prove(n, tables, nodes, consts, claimed, domain, zerocheck=False, threads=1):
+    """the oracle's proof; o["state"] is its final transcript state"""
     st = co.transcript_new(domain)
     o = co.sumcheck_prove(n, tables, nodes, consts, claimed, st, max_coeffs=q._lib.QZ_MAX_ROUND_COEFFS,
                           zerocheck=zerocheck, threads=threads)
+    o["state"] = st
+    return o
+
+
+def assert_matches_oracle(n, got, o, zerocheck=False):
+    """got = gpu_prove(...): every round polynomial and its length, the point, the evaluation, the state and z"""
+    sc, claim, state, z = got
     assert [p.shape[0] for p in sc.r_polys] == o["lens"].tolist()
     for j in range(n):
         assert np.array_equal(sc.r_polys[j], o["coeffs"][j][: o["lens"][j]]), f"round {j}"
     assert np.array_equal(claim.point, o["point"])
     assert np.array_equal(claim.evaluation, o["evaluation"])
-    assert state.tobytes() == st.tobytes()
+    assert state.tobytes() == o["state"].tobytes()
     if zerocheck:
         assert np.array_equal(z, o["z"])
-    return sc, claim, o
+
+
+def assert_same(ctx, n, tables, nodes, consts, claimed, domain, zerocheck=False, device_tables=False, threads=1):
+    got = gpu_prove(ctx, n, tables, nodes, consts, claimed, domain, zerocheck, device_tables)
+    o = oracle_prove(n, tables, nodes, consts, claimed, domain, zerocheck, threads)
+    assert_matches_oracle(n, got, o, zerocheck)
+    return got[0], got[1], o
 
 
 def test_reference_sumcheck_test(ctx):
@@ -349,10 +362,11 @@ def test_baseline_sizes_zerocheck_product3(ctx, n):
 
 
 def test_2_26_product3_verifier_and_mle(ctx):
-    """the upper end of north_star's range (2^16..2^26; 3 x 2 GiB of tables).  The oracle prover would take minutes, so
-    this checks the size-independent properties: the reference's verifier (sumcheck.rs:116-150) accepts the transcript
-    with the true sum and reproduces the prover's point and claim, and the claim equals the product of the tables'
-    MLE evaluations at that point (the reference's own acceptance test, sumcheck.rs:216-229)."""
+    """the upper end of north_star's range (2^16..2^26; 3 x 2 GiB of tables): every round polynomial, the point, the
+    evaluation and the transcript state against the oracle on all host cores (the device buffers are freed first), and
+    the size-independent properties: the reference's verifier (sumcheck.rs:116-150) accepts the transcript with the
+    true sum and reproduces the prover's point and claim, and the claim equals the product of the tables' MLE
+    evaluations at that point (the reference's own acceptance test, sumcheck.rs:216-229)."""
     n = 26
     bufs = [ctx.random_fr(1 << n, 2600 + t) for t in range(3)]
     store = q.VirtualPolynomialStore(n)
@@ -364,6 +378,14 @@ def test_2_26_product3_verifier_and_mle(ctx):
     true_sum = (2 * c0[0] + sum(c0[1:])) % FR  # s_0(0) + s_0(1)
     tr = q.Transcript(b"sumcheck_bench", ctx)
     sc, claim = q.SumcheckProof.prove(ctx, n, store, h, co.fr1(true_sum), tr)
+    tabs = []
+    for b in bufs:
+        tabs.append(b.download().reshape(-1, 32))
+        b.free()
+    ctx.trim()
+    nodes, consts = util.expr_product(3)
+    o = oracle_prove(n, tabs, nodes, consts, co.fr1(true_sum), b"sumcheck_bench", threads=NCPU)
+    assert_matches_oracle(n, (sc, claim, tr.state, None), o)
     coeffs = np.zeros((n, 8, 32), dtype=np.uint8)
     for j, p in enumerate(sc.r_polys):
         coeffs[j, : p.shape[0]] = p
@@ -372,8 +394,7 @@ def test_2_26_product3_verifier_and_mle(ctx):
     assert ok and np.array_equal(vp, claim.point) and np.array_equal(ve, claim.evaluation)
     assert st.tobytes() == tr.state.tobytes()
     prod = None
-    for b in bufs:
-        ev = co.mle_evaluate(b.download().reshape(-1, 32), claim.point)
-        b.free()
+    for t in tabs:
+        ev = co.mle_evaluate(t, claim.point)
         prod = ev if prod is None else co.field_op(0, 2, prod, ev)
     assert np.array_equal(prod.reshape(32), claim.evaluation)
