@@ -136,7 +136,6 @@ struct qz_ctx {
   }
   float last_ms[2] = {0.f, 0.f};
   double last_stat[4] = {0, 0, 0, 0};  // last MSM: window bits, digits per scalar, shared bucket set (0/1), mixed additions
-  float kernel_ms_accum = 0.f;
 
   // pinned staging for small results
   void* pinned = nullptr;

@@ -93,39 +93,23 @@ __constant__ uint32_t c_fold[64];
 QZ_DEV Fr fold_fixed(const Fr& lo, const Fr& hi) {
   return fp_add<FrParams>(lo, fp_mul_fixed<FrParams>(fp_sub_lazy<FrParams>(hi, lo), c_fold));
 }
-
-// fetch pair p of table t, folding the pending challenge first when `fold` (sumcheck.rs:81-92 fused into the next
-// round's pass): lo' = a0 + r (a1 - a0), hi' = a2 + r (a3 - a2), both written to the half-size table.
-template <bool CV = false, bool CF = false>
-QZ_DEV void fetch_pair(const uint4* in, uint4* out, uint64_t p, bool fold, const Fr& r, Fr& lo, Fr& hi) {
-  if (fold) {
-    Fr a0 = ld_elem_t<CV>(in, 4 * p), a1 = ld_elem_t<CV>(in, 4 * p + 1), a2 = ld_elem_t<CV>(in, 4 * p + 2), a3 = ld_elem_t<CV>(in, 4 * p + 3);
-    if (CF) {
-      lo = fold_fixed(a0, a1);
-      hi = fold_fixed(a2, a3);
-    } else {
-      lo = fp_add<FrParams>(a0, fp_mul<FrParams>(r, fp_sub<FrParams>(a1, a0)));
-      hi = fp_add<FrParams>(a2, fp_mul<FrParams>(r, fp_sub<FrParams>(a3, a2)));
-    }
-    st_elem(out, 2 * p, lo);
-    st_elem(out, 2 * p + 1, hi);
-  } else {
-    lo = ld_elem_t<CV>(in, 2 * p);
-    hi = ld_elem_t<CV>(in, 2 * p + 1);
-  }
+// lo + r (hi - lo) with r in registers
+QZ_DEV Fr fold_by(const Fr& lo, const Fr& hi, const Fr& r) {
+  return fp_add<FrParams>(lo, fp_mul<FrParams>(r, fp_sub<FrParams>(hi, lo)));
 }
 
-// The same in two steps for the streaming kernels: all loads of a pair are issued before any arithmetic so that one
-// memory round trip, not one per table, is exposed per pair (FOLD is a compile-time flag there: no branch splits the
-// block the scheduler can hoist loads across).
+// Pair p of a table, folding the pending challenge first when FOLD (sumcheck.rs:81-92 fused into the next round's
+// pass): lo' = a0 + r (a1 - a0), hi' = a2 + r (a3 - a2), both written to the half-size table.  In two steps so that
+// the streaming kernels issue all loads of a pair before any arithmetic: one memory round trip, not one per table, is
+// exposed per pair (FOLD is a compile-time flag there: no branch splits the block the scheduler can hoist loads across).
 template <bool FOLD>
 struct RawPair {
   Fr e[FOLD ? 4 : 2];
 };
-template <bool FOLD>
+template <bool FOLD, bool CV = false>
 QZ_DEV void load_raw(const uint4* in, uint64_t p, RawPair<FOLD>& raw) {
 #pragma unroll
-  for (int j = 0; j < (FOLD ? 4 : 2); j++) raw.e[j] = ld_elem(in, (FOLD ? 4 : 2) * p + j);
+  for (int j = 0; j < (FOLD ? 4 : 2); j++) raw.e[j] = ld_elem_t<CV>(in, (FOLD ? 4 : 2) * p + j);
 }
 template <bool FOLD, bool CF = false>
 QZ_DEV void finish_pair(const RawPair<FOLD>& raw, uint4* out, uint64_t p, const Fr& r, Fr& lo, Fr& hi) {
@@ -134,14 +118,27 @@ QZ_DEV void finish_pair(const RawPair<FOLD>& raw, uint4* out, uint64_t p, const 
       lo = fold_fixed(raw.e[0], raw.e[1]);
       hi = fold_fixed(raw.e[FOLD ? 2 : 0], raw.e[FOLD ? 3 : 1]);
     } else {
-      lo = fp_add<FrParams>(raw.e[0], fp_mul<FrParams>(r, fp_sub<FrParams>(raw.e[1], raw.e[0])));
-      hi = fp_add<FrParams>(raw.e[FOLD ? 2 : 0], fp_mul<FrParams>(r, fp_sub<FrParams>(raw.e[FOLD ? 3 : 1], raw.e[FOLD ? 2 : 0])));
+      lo = fold_by(raw.e[0], raw.e[1], r);
+      hi = fold_by(raw.e[FOLD ? 2 : 0], raw.e[FOLD ? 3 : 1], r);
     }
     st_elem(out, 2 * p, lo);
     st_elem(out, 2 * p + 1, hi);
   } else {
     lo = raw.e[0];
     hi = raw.e[1];
+  }
+}
+// the same with `fold` a run-time flag (the tail kernels)
+template <bool CV = false, bool CF = false>
+QZ_DEV void fetch_pair(const uint4* in, uint4* out, uint64_t p, bool fold, const Fr& r, Fr& lo, Fr& hi) {
+  if (fold) {
+    RawPair<true> raw;
+    load_raw<true, CV>(in, p, raw);
+    finish_pair<true, CF>(raw, out, p, r, lo, hi);
+  } else {
+    RawPair<false> raw;
+    load_raw<false, CV>(in, p, raw);
+    finish_pair<false>(raw, out, p, r, lo, hi);
   }
 }
 
@@ -419,6 +416,27 @@ __global__ void __launch_bounds__(SC_THREADS) sc_round_generic(ScTables tabs, ui
 }
 
 // ---- finalize: sum `n_parts` partial vectors, close the round (transcript on the device) -----------------------------------
+// this thread's share of the sum of the n_parts vectors of ns values in `partials` (block_sum_many adds the shares)
+QZ_DEV void sum_partials(const Fr* partials, int n_parts, int ns, Fr* v) {
+  for (int x = 0; x < ns; x++) v[x] = fp_zero<FrParams>();
+  for (int b = threadIdx.x; b < n_parts; b += blockDim.x)
+    for (int x = 0; x < ns; x++) v[x] = fp_add<FrParams>(v[x], partials[(size_t)b * ns + x]);
+}
+
+// Sharded rounds with peer mailboxes (comm.cuh): this rank's ns sums in s_evals go to every rank's mailbox over NVLink,
+// and s_evals[x] <- the sum of the G vectors addressed to this rank (field addition is exact, so the order does not
+// matter): every rank runs the same transcript on the same sums and draws the same challenge.  Ends with a barrier.
+QZ_DEV void peer_sum(PeerMailbox* const* peers, int rank, int G, uint32_t seq, ScHead* head, Fr* s_evals, int ns) {
+  const PeerSlot* got = peer_exchange(peers, rank, G, seq, s_evals, ns);
+  if (threadIdx.x == 0 && *reinterpret_cast<volatile uint32_t*>(&peers[rank]->timed_out)) head->peer_fault = 1;
+  if ((int)threadIdx.x < ns) {
+    Fr sum = fp_zero<FrParams>();
+    for (int g = 0; g < G; g++) sum = fp_add<FrParams>(sum, ld_fresh(&got->data[g][threadIdx.x]));
+    s_evals[threadIdx.x] = sum;
+  }
+  __syncthreads();
+}
+
 // derive1: the partial vectors hold ns = d sums (X = 0, 2, .., d); X = 1 is restored from the running claim
 // (sc_expand_evals).  zc_zinv: 1 / z_j for that step on the eq-factored zero-check path.
 __global__ void __launch_bounds__(SC_THREADS) sc_finalize(const Fr* partials, int n_parts, int d, ScHead* head,
@@ -434,9 +452,7 @@ __global__ void __launch_bounds__(SC_THREADS) sc_finalize(const Fr* partials, in
   grid_dep_wait();
   const int ns = derive1 ? d : d + 1;
   Fr v[SC_MAX_COEFFS];
-  for (int x = 0; x < ns; x++) v[x] = fp_zero<FrParams>();
-  for (int b = threadIdx.x; b < n_parts; b += blockDim.x)
-    for (int x = 0; x < ns; x++) v[x] = fp_add<FrParams>(v[x], partials[(size_t)b * ns + x]);
+  sum_partials(partials, n_parts, ns, v);
   block_sum_many(v, ns, s_part, s_evals);
   if (derive1) sc_expand_evals(head, d, s_evals, zc_z, zc_zinv);
   if (toom) sc_toom3_to_coeffs(s_evals);  // the sums are samples at X = 0, 1, -1, inf (prod_core_toom3)
@@ -444,10 +460,8 @@ __global__ void __launch_bounds__(SC_THREADS) sc_finalize(const Fr* partials, in
                  max_coeffs, zc_z, true, foldc);
 }
 
-// Sharded mode with peer mailboxes (comm.cuh): ONE launch per round after the round kernel.  The block sums this rank's
-// partials, stores the (d+1)-vector into every rank's mailbox over NVLink, waits for the G vectors addressed to it,
-// adds them (field addition is exact, so the order does not matter) and closes the round -- every rank runs the same
-// transcript on the same sums and draws the same challenge.  Replaces sc_reduce_partials + ncclAllGather + sc_finalize.
+// Sharded mode with peer mailboxes: ONE launch per round after the round kernel, in place of sc_reduce_partials +
+// ncclAllGather + sc_finalize.
 __global__ void __launch_bounds__(SC_THREADS) sc_finalize_peers(const Fr* partials, int n_parts, int d,
                                                                PeerMailbox* const* peers, int rank, int G, uint32_t seq,
                                                                ScHead* head, const Fr* vinv, Fr* out_coeffs_row,
@@ -463,18 +477,9 @@ __global__ void __launch_bounds__(SC_THREADS) sc_finalize_peers(const Fr* partia
   grid_dep_wait();
   const int ns = derive1 ? d : d + 1;
   Fr v[SC_MAX_COEFFS];
-  for (int x = 0; x < ns; x++) v[x] = fp_zero<FrParams>();
-  for (int b = threadIdx.x; b < n_parts; b += blockDim.x)
-    for (int x = 0; x < ns; x++) v[x] = fp_add<FrParams>(v[x], partials[(size_t)b * ns + x]);
+  sum_partials(partials, n_parts, ns, v);
   block_sum_many(v, ns, s_part, s_evals);
-  const PeerSlot* got = peer_exchange(peers, rank, G, seq, s_evals, ns);
-  if (threadIdx.x == 0 && *reinterpret_cast<volatile uint32_t*>(&peers[rank]->timed_out)) head->peer_fault = 1;
-  if ((int)threadIdx.x < ns) {
-    Fr sum = fp_zero<FrParams>();
-    for (int g = 0; g < G; g++) sum = fp_add<FrParams>(sum, ld_fresh(&got->data[g][threadIdx.x]));
-    s_evals[threadIdx.x] = sum;
-  }
-  __syncthreads();
+  peer_sum(peers, rank, G, seq, head, s_evals, ns);
   if (derive1) sc_expand_evals(head, d, s_evals, zc_z, zc_zinv);
   if (toom) sc_toom3_to_coeffs(s_evals);
   sc_round_close(head, toom ? nullptr : vinv, d, s_evals, s_coef, s_msg, s_prod, out_coeffs_row, out_len, out_point_slot,
@@ -485,9 +490,7 @@ __global__ void __launch_bounds__(SC_THREADS) sc_finalize_peers(const Fr* partia
 __global__ void __launch_bounds__(SC_THREADS) sc_reduce_partials(const Fr* partials, int n_parts, int d, Fr* out) {
   __shared__ Fr s_part[(SC_THREADS / 32) * SC_MAX_COEFFS];
   Fr v[SC_MAX_COEFFS];
-  for (int x = 0; x <= d; x++) v[x] = fp_zero<FrParams>();
-  for (int b = threadIdx.x; b < n_parts; b += blockDim.x)
-    for (int x = 0; x <= d; x++) v[x] = fp_add<FrParams>(v[x], partials[(size_t)b * (d + 1) + x]);
+  sum_partials(partials, n_parts, d + 1, v);
   block_sum_many(v, d + 1, s_part, out);
 }
 
@@ -624,8 +627,7 @@ QZ_DEV void mid_split_pass(const ScTables& view, uint64_t p_begin, uint64_t p_en
       const uint64_t idx = 2 * tile + (uint64_t)fe;             // element of the tables this round sums over
       Fr v;
       if (fold) {
-        const Fr a0 = ld_elem_cv(view.in[ft], 2 * idx), a1 = ld_elem_cv(view.in[ft], 2 * idx + 1);
-        v = fp_add<FrParams>(a0, fp_mul<FrParams>(r, fp_sub<FrParams>(a1, a0)));
+        v = fold_by(ld_elem_cv(view.in[ft], 2 * idx), ld_elem_cv(view.in[ft], 2 * idx + 1), r);
         st_elem(view.out[ft], idx, v);
       } else {
         v = ld_elem_cv(view.in[ft], idx);
@@ -831,16 +833,7 @@ __global__ void __launch_bounds__(SC_THREADS) sc_mid(ScTables tabs, ScTailBufs b
     }
     SC_TRACE(3);
     if (closer) {
-      if (!gathered) {  // sharded: all ranks' vectors (comm.cuh), exact field addition in any order
-        const PeerSlot* got = peer_exchange(peers, rank, G, seq, s_evals, ns);
-        if (threadIdx.x == 0 && *reinterpret_cast<volatile uint32_t*>(&peers[rank]->timed_out)) head->peer_fault = 1;
-        if ((int)threadIdx.x < ns) {
-          Fr sum = fp_zero<FrParams>();
-          for (int g = 0; g < G; g++) sum = fp_add<FrParams>(sum, ld_fresh(&got->data[g][threadIdx.x]));
-          s_evals[threadIdx.x] = sum;
-        }
-        __syncthreads();
-      }
+      if (!gathered) peer_sum(peers, rank, G, seq, head, s_evals, ns);
       SC_TRACE(4);
       if (skip1) sc_expand_evals(head, d, s_evals, nullptr, nullptr);
       // The other blocks are released as soon as the challenge is out, provided this block works on the next round too:
@@ -877,10 +870,7 @@ __global__ void __launch_bounds__(SC_THREADS) sc_mid(ScTables tabs, ScTailBufs b
     const Fr r = fr_ld_cv(&head->r);
     for (int t = 0; t < k; t++) {
       Fr lo = ld_elem_cv(view.in[t], 0);
-      if (pending_fold && size == 2) {
-        const Fr hi = ld_elem_cv(view.in[t], 1);
-        lo = fp_add<FrParams>(lo, fp_mul<FrParams>(r, fp_sub<FrParams>(hi, lo)));
-      }
+      if (pending_fold && size == 2) lo = fold_by(lo, ld_elem_cv(view.in[t], 1), r);
       fin[t] = lo;
     }
     Fr ev = sc_eval_program(s_ops, n_ops, consts, fin);
@@ -1005,18 +995,6 @@ __global__ void __launch_bounds__(256) eq_expand(const Fr* lo_tab, const Fr* hi_
     const uint64_t g = base + i;
     st_elem(out, i, fp_mul<FrParams>(lo_tab[g & mask], hi_tab[g >> a]));
   }
-}
-// zerocheck.rs:34-40: evaluation <- evaluation / eq_eval(z, point)
-__global__ void zc_finish(ScHead* head, const Fr* z, const Fr* point, int n) {
-  const Fr one = fp_one<FrParams>();
-  Fr e = one;
-  for (int i = 0; i < n; i++) {  // eq_eval.rs:33-43
-    Fr x = z[i], r = point[i];
-    Fr term = fp_add<FrParams>(fp_mul<FrParams>(x, r),
-                               fp_mul<FrParams>(fp_sub<FrParams>(one, x), fp_sub<FrParams>(one, r)));
-    e = fp_mul<FrParams>(e, term);
-  }
-  head->evaluation = fp_mul<FrParams>(head->evaluation, fp_inv_serial<FrParams>(e));
 }
 // Inverse Vandermonde on nodes 0..d: vinv[i*(d+1)+j] = coefficient of X^i in the Lagrange basis polynomial L_j
 __global__ void sc_build_vinv(int d, Fr* vinv) {
@@ -1223,11 +1201,47 @@ int round_grid(qz_ctx* ctx, uint64_t n_pairs, int blocks_per_sm, int threads = S
   return (int)std::max<uint64_t>(1, std::min(want, cap));
 }
 
+// resident blocks per SM of a proof's streaming-round kernels: the narrow one (at least 1) and the deferred-reduction one
+// (0: there is none).  zc: the zero-check fast path's kernels of nf factors; otherwise the product kernels of nf
+// factors, or the interpreter for nf = 0.  The folding instance stands for its family.
+struct RoundOcc {
+  int narrow, wide;
+};
+RoundOcc round_occupancy(qz_ctx* ctx, bool zc, int nf) {
+  RoundOcc o = {1, 0};
+  if (zc) {
+    if (nf == 1) o.narrow = blocks_per_sm(ctx, sc_round_zc<1, false, true, false>, SC_THREADS);
+    else if (nf == 2) o.narrow = blocks_per_sm(ctx, sc_round_zc<2, false, true, false>, SC_THREADS);
+    else {
+      o.narrow = blocks_per_sm(ctx, sc_round_zc<3, false, true, false>, SC_THREADS);
+      o.wide = blocks_per_sm(ctx, sc_round_zc<3, true, true, false>, SC_WIDE_THREADS);
+    }
+  } else if (nf == 1) {
+    o.narrow = blocks_per_sm(ctx, sc_round_prod<1, false, true>, SC_THREADS);
+  } else if (nf == 2) {
+    o.narrow = blocks_per_sm(ctx, sc_round_prod<2, false, true>, SC_THREADS);
+  } else if (nf == 3) {
+    o.narrow = blocks_per_sm(ctx, sc_round_prod<3, false, true>, SC_THREADS);
+    o.wide = blocks_per_sm(ctx, sc_round_prod<3, true, true>, SC_WIDE_THREADS);
+  } else if (nf == 4) {
+    o.narrow = blocks_per_sm(ctx, sc_round_prod<4, false, true>, SC_THREADS);
+    o.wide = blocks_per_sm(ctx, sc_round_prod<4, true, true>, SC_WIDE_THREADS);
+  } else {
+    o.narrow = blocks_per_sm(ctx, sc_round_generic<true>, SC_THREADS);
+  }
+  o.narrow = std::max(o.narrow, 1);
+  return o;
+}
+// a streaming round's kernel variant and grid
+struct RoundShape {
+  bool wide;
+  int grid;
+};
+
 }  // namespace
 
 namespace qz {
 
-static thread_local bool tl_zc_no_skip = false;  // set while a zero-check is redone without the SKIP1 rounds
 // c_fold is one table per device: proofs of different contexts on the same device take turns
 static std::recursive_mutex g_fold_table_lock[16];
 
@@ -1338,11 +1352,12 @@ int logup_denominators_run(qz_ctx* ctx, size_t num_vars, size_t k, const void* c
 
 // The whole proof.  `sharded`: `tables` hold this rank's contiguous shard, elements [rank * 2^num_vars / nranks, ...),
 // i.e. the tables are split by the top variables so every (2p, 2p+1) pair is local (sumcheck.rs:56-57).
-int sumcheck_run(qz_ctx* ctx, size_t num_vars, size_t k, const void* const* tables, int tables_on_device,
-                 const qz_expr_node* nodes, size_t n_nodes, const uint8_t* consts, size_t n_consts,
-                 const uint8_t* claimed_sum, uint8_t* state, size_t max_coeffs, uint8_t* out_coeffs,
-                 uint32_t* out_lens, uint8_t* out_point, uint8_t* out_eval, bool zerocheck, uint8_t* out_z,
-                 bool sharded) {
+// allow_zc_skip1 false: a zero-check runs without the SKIP1 rounds (the redo after some z_j = 0).
+static int sumcheck_prove(qz_ctx* ctx, size_t num_vars, size_t k, const void* const* tables, int tables_on_device,
+                          const qz_expr_node* nodes, size_t n_nodes, const uint8_t* consts, size_t n_consts,
+                          const uint8_t* claimed_sum, uint8_t* state, size_t max_coeffs, uint8_t* out_coeffs,
+                          uint32_t* out_lens, uint8_t* out_point, uint8_t* out_eval, bool zerocheck, uint8_t* out_z,
+                          bool sharded, bool allow_zc_skip1) {
   if (!ctx || !state || !out_eval || (num_vars && (!out_coeffs || !out_lens || !out_point)))
     return ctx ? ctx->fail(QZ_ERR_INVALID_ARG, "null pointer") : QZ_ERR_INVALID_ARG;
   if (num_vars > (size_t)SC_MAX_VARS - 1 || (k && !tables) || (n_nodes && !nodes) || (n_consts && !consts))
@@ -1401,25 +1416,36 @@ int sumcheck_run(qz_ctx* ctx, size_t num_vars, size_t k, const void* const* tabl
     memcpy(pin + in_consts, consts, 32 * n_consts);
     QZ_CUDA(ctx, cudaMemcpyAsync(d_in + in_consts, pin + in_consts, 32 * n_consts, cudaMemcpyHostToDevice, st));
   }
-  bool zc_skip1 = false;
+
+  // streaming rounds run while a rank's table has more than 2^SC_MID_LOG entries (with peer mailboxes or one GPU; the
+  // NCCL fallback streams down to the gather size), then sc_mid takes every remaining round
+  const bool mid_sharded = G == 1 || comm_has_peers(ctx);
+  static const int mid_log = [] {  // QZ_SC_MID_LOG: measurement switch for the hand-over size (DESIGN.md section 10)
+    const char* e = getenv("QZ_SC_MID_LOG");
+    const int v = e ? atoi(e) : SC_MID_LOG;
+    return v >= SC_TAIL_LOG && v <= 24 ? v : SC_MID_LOG;
+  }();
+  auto streaming = [&](uint64_t sz) {
+    return mid_sharded ? sz > ((uint64_t)1 << mid_log) : sz * G > ((uint64_t)1 << SC_TAIL_LOG);
+  };
+  // zero-check fast path (see sc_round_zc): h is a product of up to three tables and at least one streaming round runs.
+  // From 2^21 entries on it skips X = 1 from round 1 on, which repays the batched inversion of the z in sc_begin
+  // (~30 us on one thread).
+  const bool zc_fast =
+      zerocheck && cp.product_k >= 2 && cp.product_k <= 4 && streaming(N) && !getenv("QZ_ZC_STREAM_EQ");
+  const bool zc_skip1 = zc_fast && num_vars >= 21 && allow_zc_skip1 && !getenv("QZ_ZC_NO_SKIP1");
   Fr* d_zinv = nullptr;
-  ScMidSync* d_sync = nullptr;
-  uint32_t* d_foldc = nullptr;  // multiples of the last challenge (sc_round_close), copied into c_fold before a large fold pass
+  if (zc_skip1) {
+    d_zinv = (Fr*)ctx->arena_alloc(32 * num_vars);
+    if (!d_zinv) return ctx->fail(QZ_ERR_ALLOC, "zero-check inverses");
+  }
+  ScMidSync* d_sync = (ScMidSync*)ctx->arena_alloc(sizeof(ScMidSync));
+  uint32_t* d_foldc = (uint32_t*)ctx->arena_alloc(64 * sizeof(uint32_t));  // multiples of the last challenge (sc_round_close)
+  if (!d_sync || !d_foldc) return ctx->fail(QZ_ERR_ALLOC, "round counters");
   {
     Fr cs;
     memset(&cs, 0, sizeof cs);
     if (!zerocheck) memcpy(cs.v, claimed_sum, 32);
-    // the eq-factored zero-check skips X = 1 from round 1 on when the proof is large enough to repay the batched
-    // inversion of the z (~30 us on one thread); decided here because sc_begin computes the inverses
-    const bool zc_maybe_fast = zerocheck && cp.product_k >= 2 && cp.product_k <= 4 && !getenv("QZ_ZC_STREAM_EQ");
-    zc_skip1 = zc_maybe_fast && num_vars >= 21 && !tl_zc_no_skip && !getenv("QZ_ZC_NO_SKIP1");
-    if (zc_skip1) {
-      d_zinv = (Fr*)ctx->arena_alloc(32 * num_vars);
-      if (!d_zinv) return ctx->fail(QZ_ERR_ALLOC, "zero-check inverses");
-    }
-    d_sync = (ScMidSync*)ctx->arena_alloc(sizeof(ScMidSync));
-    d_foldc = (uint32_t*)ctx->arena_alloc(64 * sizeof(uint32_t));
-    if (!d_sync || !d_foldc) return ctx->fail(QZ_ERR_ALLOC, "round counters");
     ScStateArg state_arg;
     memcpy(state_arg.b, state, 32);
     QZ_LAUNCH(ctx, sc_begin, 1, 32, 0, head, state_arg, (uint64_t)num_vars, cs, zerocheck ? (int)num_vars : 0, d_z, d_zinv,
@@ -1436,7 +1462,8 @@ int sumcheck_run(qz_ctx* ctx, size_t num_vars, size_t k, const void* const* tabl
   uint8_t* up_dst[SC_MAX_K];
   const uint8_t* up_src[SC_MAX_K];
   int n_up = 0;
-  // tables referenced by h: device copies (host input) or the caller's device buffers
+  // tables referenced by h: device copies (host input) or the caller's device buffers.  A zero-check always has the eq
+  // slot: h_hat's root multiplies by it.
   ScTables tabs;
   memset(&tabs, 0, sizeof tabs);
   int eq_slot = -1;
@@ -1461,21 +1488,7 @@ int sumcheck_run(qz_ctx* ctx, size_t num_vars, size_t k, const void* const* tabl
       tabs.in[j] = (const uint4*)p;
     }
   }
-  // zero-check fast path (see sc_round_zc): h is a product of up to three tables and at least one streaming round runs
-  // streaming rounds run while a rank's table has more than 2^SC_MID_LOG entries (with peer mailboxes or one GPU; the
-  // NCCL fallback streams down to the gather size), then sc_mid takes every remaining round
-  const bool mid_sharded = G == 1 || comm_has_peers(ctx);
-  static const int mid_log = [] {  // QZ_SC_MID_LOG: measurement switch for the hand-over size (DESIGN.md section 10)
-    const char* e = getenv("QZ_SC_MID_LOG");
-    const int v = e ? atoi(e) : SC_MID_LOG;
-    return v >= SC_TAIL_LOG && v <= 24 ? v : SC_MID_LOG;
-  }();
-  auto streaming = [&](uint64_t sz) {
-    return mid_sharded ? sz > ((uint64_t)1 << mid_log) : sz * G > ((uint64_t)1 << SC_TAIL_LOG);
-  };
-  const bool zc_fast = zerocheck && eq_slot >= 0 && cp.product_k >= 2 && cp.product_k <= 4 && streaming(N) &&
-                       !getenv("QZ_ZC_STREAM_EQ");
-  if (zerocheck && eq_slot >= 0 && !zc_fast) {
+  if (zerocheck && !zc_fast) {
     void* p = ctx->arena_alloc(32 * N);
     if (!p) return ctx->fail(QZ_ERR_ALLOC, "eq table");
     rc = eq_table_device(ctx, (int)num_vars, d_z, (uint4*)p, (uint64_t)ctx->rank * N * (G > 1), N);  // zerocheck.rs:25
@@ -1494,154 +1507,106 @@ int sumcheck_run(qz_ctx* ctx, size_t num_vars, size_t k, const void* const* tabl
       bufB[j] = (uint4*)ctx->arena_alloc(32 * std::max<uint64_t>(1, N / 4));
       if (!bufA[j] || !bufB[j]) return ctx->fail(QZ_ERR_ALLOC, "fold scratch");
     }
-    // occupancy-sized grids for the streaming rounds
-    int bps = 1;
-    int bps_wide = 0;  // > 0: a deferred-reduction variant of the round kernel exists for this product
-    if (cp.product_k == 1) bps = blocks_per_sm(ctx, sc_round_prod<1, false, true>, SC_THREADS);
-    else if (cp.product_k == 2) bps = blocks_per_sm(ctx, sc_round_prod<2, false, true>, SC_THREADS);
-    else if (cp.product_k == 3) {
-      bps = blocks_per_sm(ctx, sc_round_prod<3, false, true>, SC_THREADS);
-      bps_wide = blocks_per_sm(ctx, sc_round_prod<3, true, true>, SC_WIDE_THREADS);
-    } else if (cp.product_k == 4) {
-      bps = blocks_per_sm(ctx, sc_round_prod<4, false, true>, SC_THREADS);
-      bps_wide = blocks_per_sm(ctx, sc_round_prod<4, true, true>, SC_WIDE_THREADS);
-    } else bps = blocks_per_sm(ctx, sc_round_generic<true>, SC_THREADS);
-    if (bps < 1) bps = 1;
-    if (getenv("QZ_SC_NARROW")) bps_wide = 0;  // measurement switch: force the fully reduced sums
-    Fr* partials = (Fr*)ctx->arena_alloc(sizeof(Fr) * std::max<size_t>((size_t)ctx->sm_count * std::max(bps, bps_wide), SC_THREADS) * (d + 1) * up_chunks);
+    // The streaming rounds fold the nt tables ft.in[i] = tabs.in[slot_of[i]]: every table of h, or on the zero-check
+    // fast path the K tables of h without the eq slot, whose fold scratch holds the weight tables instead.  nf: factors
+    // of the round kernel's product (0: the interpreter); deg, vinv_r: degree and interpolation matrix of the sums.
+    const int nf = zc_fast ? cp.product_k - 1 : cp.product_k, deg = zc_fast ? nf : d;
+    Fr* vinv_r = vinv;
+    if (zc_fast) {
+      rc = get_vinv(ctx, deg, &vinv_r);
+      if (rc) return rc;
+    }
+    ScTables ft;
+    memset(&ft, 0, sizeof ft);
+    int slot_of[SC_MAX_K], nt = 0;
+    for (int j = 0; j < ka; j++)
+      if (!zc_fast || j != eq_slot) {
+        ft.in[nt] = tabs.in[j];
+        slot_of[nt++] = j;
+      }
+    // occupancy-sized grids.  `partials` holds a vector per block of the product kernel of all of h's tables; the
+    // zero-check fast path's kernels are capped at that many blocks per SM.
+    const bool narrow_only = getenv("QZ_SC_NARROW") != nullptr;  // measurement switch: force the fully reduced sums
+    RoundOcc occ = round_occupancy(ctx, false, cp.product_k);
+    if (narrow_only) occ.wide = 0;
+    const int part_bps = std::max(occ.narrow, occ.wide);
+    if (zc_fast) {
+      const RoundOcc z = round_occupancy(ctx, true, nf);
+      occ = {std::min(z.narrow, part_bps), narrow_only ? 0 : std::min(z.wide, part_bps)};
+    }
+    // deferred reduction pays once a thread sums several pairs (its one-off reduction is 3 products per sum)
+    auto pick = [&](uint64_t n_pairs) {
+      RoundShape s;
+      s.wide = occ.wide > 0 && n_pairs >= (uint64_t)8 * SC_WIDE_THREADS * ctx->sm_count * occ.wide;
+      s.grid = s.wide ? round_grid(ctx, n_pairs, occ.wide, SC_WIDE_THREADS) : round_grid(ctx, n_pairs, occ.narrow);
+      return s;
+    };
+    Fr* partials = (Fr*)ctx->arena_alloc(sizeof(Fr) * std::max<size_t>((size_t)ctx->sm_count * part_bps, SC_THREADS) * (d + 1) * up_chunks);
     Fr* rank_evals = (Fr*)ctx->arena_alloc(sizeof(Fr) * (d + 1));
     Fr* all_evals = (Fr*)ctx->arena_alloc(sizeof(Fr) * (size_t)(d + 1) * G);
     if (!partials || !rank_evals || !all_evals) return ctx->fail(QZ_ERR_ALLOC, "partials");
 
     uint64_t size = N;  // current (pre-fold) table size
     int pending = 0, round = 0, flip = 0;
-    const uint4* zc_weights = nullptr;  // zero-check fast path: E_j, the weight table of the last round run (size / 2 entries)
     // the round chain uses programmatic dependent launches, except around NCCL collectives (not written for them)
     // Measured (tools/sc_pdl_ab.py): -5 us per round while a round is latency-bound,
     // but +10..20 us on the rounds that stream 2^21 entries or more, so only the short rounds are chained this way.
     const bool pdl_ok = ctx->pdl && (G == 1 || comm_has_peers(ctx));
-    ctx->kernel_ms_accum = 0.f;
     std::unique_ptr<QzRange> nvtx_stream(new QzRange("qz:sumcheck:streaming-rounds"));
     QZ_CUDA(ctx, cudaEventRecord(ctx->ev_k0, st));
+    // zero-check fast path: E_j, the weight table of round j, ping-pongs between the eq slot's fold scratch; E_1 = eq
+    // table of z_1 .. z_{n-1}, this rank's N/2 entries
+    uint4* e_buf[2] = {nullptr, nullptr};
+    int e_cur = 0;
     if (zc_fast) {
-      const int K = cp.product_k - 1;  // factors of h; the eq factor is carried by the weights
-      Fr* vinv_k = nullptr;
-      rc = get_vinv(ctx, K, &vinv_k);
-      if (rc) return rc;
-      int zb = 1, zb_wide = 0;
-      if (K == 1) zb = blocks_per_sm(ctx, sc_round_zc<1, false, true, false>, SC_THREADS);
-      else if (K == 2) zb = blocks_per_sm(ctx, sc_round_zc<2, false, true, false>, SC_THREADS);
-      else {
-        zb = blocks_per_sm(ctx, sc_round_zc<3, false, true, false>, SC_THREADS);
-        zb_wide = blocks_per_sm(ctx, sc_round_zc<3, true, true, false>, SC_WIDE_THREADS);
-      }
-      zb = std::max(1, std::min(zb, std::max(bps, bps_wide)));  // `partials` was sized for max(bps, bps_wide) blocks per SM
-      zb_wide = std::min(zb_wide, std::max(bps, bps_wide));
-      if (getenv("QZ_SC_NARROW")) zb_wide = 0;
-      // the eq slot's fold scratch holds the weight tables: E_1 = eq table of z_1 .. z_{n-1}, this rank's N/2 entries
-      uint4* e_buf[2] = {bufA[eq_slot], bufB[eq_slot]};
+      e_buf[0] = bufA[eq_slot];
+      e_buf[1] = bufB[eq_slot];
       rc = eq_table_device(ctx, (int)num_vars - 1, d_z + 1, e_buf[0], (uint64_t)ctx->rank * (N / 2) * (G > 1), N / 2);
       if (rc) return rc;
-      int e_cur = 0;
-      ScTables gt;  // the K tables of h, in dense order without the eq slot
-      memset(&gt, 0, sizeof gt);
-      int g_of[SC_MAX_K];
-      for (int j = 0, i = 0; j < ka; j++)
-        if (j != eq_slot) {
-          gt.in[i] = tabs.in[j];
-          g_of[i++] = j;
-        }
-      while (streaming(size)) {
-        const uint64_t n_pairs = pending ? size / 4 : size / 2;
-        const bool pdl = pdl_ok && n_pairs <= ((uint64_t)1 << 18);
-        for (int i = 0; i < K; i++) gt.out[i] = flip ? bufB[g_of[i]] : bufA[g_of[i]];
-        const bool wide = zb_wide > 0 && n_pairs >= (uint64_t)8 * SC_WIDE_THREADS * ctx->sm_count * zb_wide;
-        int grid = wide ? round_grid(ctx, n_pairs, zb_wide, SC_WIDE_THREADS) : round_grid(ctx, n_pairs, zb);
+    }
+    // one round kernel over `n_pairs` pairs of `tb` (fold of the pending challenge fused when `pend`)
+    const uint64_t generic_cf_pairs = (uint64_t)1 << 16;
+    auto launch_round = [&](const ScTables& tb, uint64_t n_pairs, int pend, const RoundShape& rs, bool pdl, Fr* parts) -> int {
+      const int grid = rs.grid;
+      // the deferred-reduction passes (finish_pair<FOLD, WIDE>) and the large interpreted ones (sc_round_generic<true>)
+      // fold through the challenge table in constant memory: bring it up to date first
+      const bool generic_cf = nf == 0 && pend && n_pairs >= generic_cf_pairs;
+      if (pend && (rs.wide || generic_cf))
+        QZ_CUDA(ctx, cudaMemcpyToSymbolAsync(c_fold, d_foldc, 64 * sizeof(uint32_t), 0, cudaMemcpyDeviceToDevice, st));
+      if (zc_fast) {
         const uint4* e_in = e_buf[e_cur];
         uint4* e_out = e_buf[e_cur ^ 1];
-
-        const int derive1 = pending && zc_skip1 ? 1 : 0;
-        if (pending && wide && K == 3)  // the deferred-reduction pass folds through c_fold
-          QZ_CUDA(ctx, cudaMemcpyToSymbolAsync(c_fold, d_foldc, 64 * sizeof(uint32_t), 0, cudaMemcpyDeviceToDevice, st));
+        const bool skip1 = pend && zc_skip1;
 #define QZ_ROUND_ZC(KK, W, T)                                                                                      \
   do {                                                                                                             \
-    if (derive1) QZ_LAUNCH_PDL(ctx, pdl, (sc_round_zc<KK, W, true, true>), grid, T, gt, e_in, e_out, n_pairs, (const ScHead*)head, partials); \
-    else if (pending) QZ_LAUNCH_PDL(ctx, pdl, (sc_round_zc<KK, W, true, false>), grid, T, gt, e_in, e_out, n_pairs, (const ScHead*)head, partials); \
-    else QZ_LAUNCH_PDL(ctx, pdl, (sc_round_zc<KK, W, false, false>), grid, T, gt, e_in, e_out, n_pairs, (const ScHead*)head, partials);        \
+    if (skip1) QZ_LAUNCH_PDL(ctx, pdl, (sc_round_zc<KK, W, true, true>), grid, T, tb, e_in, e_out, n_pairs, (const ScHead*)head, parts); \
+    else if (pend) QZ_LAUNCH_PDL(ctx, pdl, (sc_round_zc<KK, W, true, false>), grid, T, tb, e_in, e_out, n_pairs, (const ScHead*)head, parts); \
+    else QZ_LAUNCH_PDL(ctx, pdl, (sc_round_zc<KK, W, false, false>), grid, T, tb, e_in, e_out, n_pairs, (const ScHead*)head, parts);        \
   } while (0)
-        switch (K) {
+        switch (nf) {
           case 1: QZ_ROUND_ZC(1, false, SC_THREADS); break;
           case 2: QZ_ROUND_ZC(2, false, SC_THREADS); break;
           default:
-            if (wide) QZ_ROUND_ZC(3, true, SC_WIDE_THREADS);
+            if (rs.wide) QZ_ROUND_ZC(3, true, SC_WIDE_THREADS);
             else QZ_ROUND_ZC(3, false, SC_THREADS);
         }
 #undef QZ_ROUND_ZC
-        const Fr* zinv_j = zc_skip1 ? d_zinv + round : nullptr;
-        const int ns = derive1 ? K : K + 1;
-        const int toom = wide && K == 3 ? 1 : 0;  // the sums are samples at X = 0, 1, -1, inf (prod_core_toom3)
-        if (G == 1) {
-          QZ_LAUNCH_PDL(ctx, pdl, sc_finalize, 1, SC_THREADS, (const Fr*)partials, grid, K, head, (const Fr*)vinv_k,
-                        d_coeffs + (size_t)round * mc, d_lens + round, d_point + round, mc, (const Fr*)(d_z + round), derive1,
-                        zinv_j, d_foldc, toom);
-        } else if (comm_has_peers(ctx)) {
-          QZ_LAUNCH_PDL(ctx, pdl, sc_finalize_peers, 1, SC_THREADS, (const Fr*)partials, grid, K,
-                        (PeerMailbox* const*)ctx->peer_mbox_dev, ctx->rank, G, ++ctx->mbox_seq, head, (const Fr*)vinv_k,
-                        d_coeffs + (size_t)round * mc, d_lens + round, d_point + round, mc, (const Fr*)(d_z + round), derive1,
-                        zinv_j, d_foldc, toom);
-        } else {
-          QZ_LAUNCH(ctx, sc_reduce_partials, 1, SC_THREADS, 0, partials, grid, ns - 1, rank_evals);
-          rc = comm_allgather(ctx, rank_evals, all_evals, sizeof(Fr) * ns);
-          if (rc) return rc;
-          QZ_LAUNCH(ctx, sc_finalize, 1, SC_THREADS, 0, all_evals, G, K, head, vinv_k, d_coeffs + (size_t)round * mc,
-                    d_lens + round, d_point + round, mc, (const Fr*)(d_z + round), derive1, zinv_j, d_foldc, toom);
-        }
-        if (pending) {
-          for (int i = 0; i < K; i++) gt.in[i] = gt.out[i];
-          flip ^= 1;
-          size >>= 1;
-          e_cur ^= 1;  // this round wrote E_{round+1} to e_out
-        }
-        zc_weights = e_buf[e_cur];
-        pending = 1;
-        round++;
-      }
-      // hand over to sc_mid: h's tables where they stand, eq materialised in the reference's form (pending fold)
-      uint4* eq_full = (uint4*)ctx->arena_alloc(32 * size);
-      if (!eq_full) return ctx->fail(QZ_ERR_ALLOC, "eq hand-over");
-      QZ_LAUNCH(ctx, zc_materialize_eq, (unsigned)((size / 2 + 255) / 256), 256, 0, zc_weights, size / 2, head,
-                (const Fr*)(d_z + (round - 1)), eq_full);
-      for (int i = 0; i < K; i++) tabs.in[g_of[i]] = gt.in[i];
-      tabs.in[eq_slot] = eq_full;
-    }
-    // one round kernel over `n_pairs` pairs of `tb` (fold of the pending challenge fused when `pend`)
-    // a pass folds through the challenge table in constant memory when it is a deferred-reduction (large) product pass
-    // or a large interpreted pass
-    const uint64_t generic_cf_pairs = (uint64_t)1 << 16;
-    auto refresh_fold_table = [&]() -> int {
-      QZ_CUDA(ctx, cudaMemcpyToSymbolAsync(c_fold, d_foldc, 64 * sizeof(uint32_t), 0, cudaMemcpyDeviceToDevice, st));
-      return QZ_OK;
-    };
-    auto launch_round = [&](const ScTables& tb, uint64_t n_pairs, int pend, int& grid, bool wide, bool pdl, Fr* parts) -> int {
-      const bool generic_cf = cp.product_k == 0 && pend && n_pairs >= generic_cf_pairs;
-      if (pend && (wide || generic_cf)) {
-        int rcf = refresh_fold_table();
-        if (rcf) return rcf;
+        return QZ_OK;
       }
 #define QZ_ROUND_PROD(K, W, T)                                                                                  \
   do {                                                                                                          \
     if (pend) QZ_LAUNCH_PDL(ctx, pdl, (sc_round_prod<K, W, true>), grid, T, tb, n_pairs, (const ScHead*)head, parts); \
     else QZ_LAUNCH_PDL(ctx, pdl, (sc_round_prod<K, W, false>), grid, T, tb, n_pairs, (const ScHead*)head, parts);     \
   } while (0)
-      switch (cp.product_k) {
+      switch (nf) {
         case 1: QZ_ROUND_PROD(1, false, SC_THREADS); break;
         case 2: QZ_ROUND_PROD(2, false, SC_THREADS); break;
         case 3:
-          if (wide) QZ_ROUND_PROD(3, true, SC_WIDE_THREADS);
+          if (rs.wide) QZ_ROUND_PROD(3, true, SC_WIDE_THREADS);
           else QZ_ROUND_PROD(3, false, SC_THREADS);
           break;
         case 4:
-          if (wide) QZ_ROUND_PROD(4, true, SC_WIDE_THREADS);
+          if (rs.wide) QZ_ROUND_PROD(4, true, SC_WIDE_THREADS);
           else QZ_ROUND_PROD(4, false, SC_THREADS);
           break;
         default:
@@ -1652,6 +1617,32 @@ int sumcheck_run(qz_ctx* ctx, size_t num_vars, size_t k, const void* const* tabl
             QZ_LAUNCH_PDL(ctx, pdl, sc_round_generic<false>, grid, SC_THREADS, tb, n_pairs, pend, (const ScHead*)head,
                           (const ScProgram*)d_prog, (const Fr*)d_consts, parts);
       }
+#undef QZ_ROUND_PROD
+      return QZ_OK;
+    };
+    // Close round `rnd` from the n_parts partial vectors in `parts` (transcript on the device): on one GPU, through the
+    // peers' mailboxes, or (NCCL fallback) by all-gathering one vector per rank, after which every rank runs the same
+    // transcript on the same sums.  Every round but the first leaves X = 1 to the running claim (ProdAcc, generic_pair).
+    auto close_round = [&](const Fr* parts, int n_parts, int rnd, int pend, bool wide, bool pdl) -> int {
+      const int derive1 = pend && (zc_fast ? zc_skip1 : d >= 1) ? 1 : 0, ns = derive1 ? deg : deg + 1;
+      const Fr* z_j = zc_fast ? d_z + rnd : nullptr;
+      const Fr* zinv_j = zc_skip1 ? d_zinv + rnd : nullptr;
+      const int toom = wide && nf == 3 ? 1 : 0;  // the sums are samples at X = 0, 1, -1, inf (prod_core_toom3)
+      Fr* coeffs = d_coeffs + (size_t)rnd * mc;
+      if (G == 1) {
+        QZ_LAUNCH_PDL(ctx, pdl, sc_finalize, 1, SC_THREADS, parts, n_parts, deg, head, (const Fr*)vinv_r, coeffs,
+                      d_lens + rnd, d_point + rnd, mc, z_j, derive1, zinv_j, d_foldc, toom);
+      } else if (comm_has_peers(ctx)) {
+        QZ_LAUNCH_PDL(ctx, pdl, sc_finalize_peers, 1, SC_THREADS, parts, n_parts, deg,
+                      (PeerMailbox* const*)ctx->peer_mbox_dev, ctx->rank, G, ++ctx->mbox_seq, head, (const Fr*)vinv_r,
+                      coeffs, d_lens + rnd, d_point + rnd, mc, z_j, derive1, zinv_j, d_foldc, toom);
+      } else {
+        QZ_LAUNCH(ctx, sc_reduce_partials, 1, SC_THREADS, 0, parts, n_parts, ns - 1, rank_evals);
+        const int rca = comm_allgather(ctx, rank_evals, all_evals, sizeof(Fr) * ns);
+        if (rca) return rca;
+        QZ_LAUNCH(ctx, sc_finalize, 1, SC_THREADS, 0, all_evals, G, deg, head, vinv_r, coeffs, d_lens + rnd,
+                  d_point + rnd, mc, z_j, derive1, zinv_j, d_foldc, toom);
+      }
       return QZ_OK;
     };
     if (up_chunks > 1) {  // round 0 behind the host -> device copies, slice by slice
@@ -1660,58 +1651,47 @@ int sumcheck_run(qz_ctx* ctx, size_t num_vars, size_t k, const void* const* tabl
       QZ_CUDA(ctx, cudaEventRecord(ctx->ev_entry, st));  // earlier users of the arena are done before the copies land
       QZ_CUDA(ctx, cudaStreamWaitEvent(ps, ctx->ev_entry, 0));
       const uint64_t per = N / up_chunks, pairs_c = per / 2;
-      const bool wide = bps_wide > 0 && pairs_c >= (uint64_t)8 * SC_WIDE_THREADS * ctx->sm_count * bps_wide;
-      int grid_c = wide ? round_grid(ctx, pairs_c, bps_wide, SC_WIDE_THREADS) : round_grid(ctx, pairs_c, bps);
+      const RoundShape rs = pick(pairs_c);
       for (int c = 0; c < up_chunks; c++) {
         for (int u = 0; u < n_up; u++)
           QZ_CUDA(ctx, cudaMemcpyAsync(up_dst[u] + 32 * per * c, up_src[u] + 32 * per * c, 32 * per, cudaMemcpyHostToDevice, ps));
         QZ_CUDA(ctx, cudaEventRecord(ctx->ev_seg_ready[c], ps));
         QZ_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev_seg_ready[c], 0));
-        ScTables slice = tabs;
-        for (int j = 0; j < ka; j++) slice.in[j] = tabs.in[j] + 2 * per * c;
-        rc = launch_round(slice, pairs_c, 0, grid_c, wide, false, partials + (size_t)c * grid_c * (d + 1));
+        ScTables slice = ft;
+        for (int i = 0; i < nt; i++) slice.in[i] = ft.in[i] + 2 * per * c;
+        rc = launch_round(slice, pairs_c, 0, rs, false, partials + (size_t)c * rs.grid * (d + 1));
         if (rc) return rc;
       }
-      QZ_LAUNCH(ctx, sc_finalize, 1, SC_THREADS, 0, (const Fr*)partials, grid_c * up_chunks, d, head, (const Fr*)vinv, d_coeffs,
-                d_lens, d_point, mc, (const Fr*)nullptr, 0, (const Fr*)nullptr, d_foldc, wide && cp.product_k == 3 ? 1 : 0);
+      rc = close_round(partials, rs.grid * up_chunks, 0, 0, rs.wide, false);
+      if (rc) return rc;
       pending = 1;
       round = 1;
     }
-    while (!zc_fast && streaming(size)) {
+    while (streaming(size)) {
       const uint64_t n_pairs = pending ? size / 4 : size / 2;
       const bool pdl = pdl_ok && n_pairs <= ((uint64_t)1 << 18);
-      for (int j = 0; j < ka; j++) tabs.out[j] = flip ? bufB[j] : bufA[j];
-      // deferred reduction pays once a thread sums several pairs (its one-off reduction is 3 products per sum)
-      const bool wide = bps_wide > 0 && n_pairs >= (uint64_t)8 * SC_WIDE_THREADS * ctx->sm_count * bps_wide;
-      int grid = wide ? round_grid(ctx, n_pairs, bps_wide, SC_WIDE_THREADS) : round_grid(ctx, n_pairs, bps);
-      rc = launch_round(tabs, n_pairs, pending, grid, wide, pdl, partials);
+      for (int i = 0; i < nt; i++) ft.out[i] = flip ? bufB[slot_of[i]] : bufA[slot_of[i]];
+      const RoundShape rs = pick(n_pairs);
+      rc = launch_round(ft, n_pairs, pending, rs, pdl, partials);
       if (rc) return rc;
-      // every round but the first leaves X = 1 to the running claim (ProdAcc / generic_pair)
-      const int derive1 = pending && d >= 1 ? 1 : 0, ns = derive1 ? d : d + 1;
-      const int toom = wide && cp.product_k == 3 ? 1 : 0;  // the sums are samples at X = 0, 1, -1, inf (prod_core_toom3)
-      if (G == 1) {
-        QZ_LAUNCH_PDL(ctx, pdl, sc_finalize, 1, SC_THREADS, (const Fr*)partials, grid, d, head, (const Fr*)vinv,
-                      d_coeffs + (size_t)round * mc, d_lens + round, d_point + round, mc, (const Fr*)nullptr, derive1,
-                      (const Fr*)nullptr, d_foldc, toom);
-      } else if (comm_has_peers(ctx)) {  // partial sums go straight into the peers' mailboxes (comm.cuh)
-        QZ_LAUNCH_PDL(ctx, pdl, sc_finalize_peers, 1, SC_THREADS, (const Fr*)partials, grid, d,
-                      (PeerMailbox* const*)ctx->peer_mbox_dev, ctx->rank, G, ++ctx->mbox_seq, head, (const Fr*)vinv,
-                      d_coeffs + (size_t)round * mc, d_lens + round, d_point + round, mc, (const Fr*)nullptr, derive1,
-                      (const Fr*)nullptr, d_foldc, toom);
-      } else {  // every rank sums all ranks' partial evaluations and runs the same transcript
-        QZ_LAUNCH(ctx, sc_reduce_partials, 1, SC_THREADS, 0, partials, grid, ns - 1, rank_evals);
-        rc = comm_allgather(ctx, rank_evals, all_evals, sizeof(Fr) * ns);
-        if (rc) return rc;
-        QZ_LAUNCH(ctx, sc_finalize, 1, SC_THREADS, 0, all_evals, G, d, head, vinv, d_coeffs + (size_t)round * mc,
-                  d_lens + round, d_point + round, mc, (const Fr*)nullptr, derive1, (const Fr*)nullptr, d_foldc, toom);
-      }
+      rc = close_round(partials, rs.grid, round, pending, rs.wide, pdl);
+      if (rc) return rc;
       if (pending) {
-        for (int j = 0; j < ka; j++) tabs.in[j] = tabs.out[j];
+        for (int i = 0; i < nt; i++) ft.in[i] = ft.out[i];
         flip ^= 1;
         size >>= 1;
+        if (zc_fast) e_cur ^= 1;  // this round wrote E_{round+1}
       }
       pending = 1;
       round++;
+    }
+    for (int i = 0; i < nt; i++) tabs.in[slot_of[i]] = ft.in[i];
+    if (zc_fast) {  // hand over to sc_mid: h's tables where they stand, eq materialised in the reference's form (pending fold)
+      uint4* eq_full = (uint4*)ctx->arena_alloc(32 * size);
+      if (!eq_full) return ctx->fail(QZ_ERR_ALLOC, "eq hand-over");
+      QZ_LAUNCH(ctx, zc_materialize_eq, (unsigned)((size / 2 + 255) / 256), 256, 0, e_buf[e_cur], size / 2, head,
+                (const Fr*)(d_z + (round - 1)), eq_full);
+      tabs.in[eq_slot] = eq_full;
     }
     QZ_CUDA(ctx, cudaEventRecord(ctx->ev_k1, st));
     nvtx_stream.reset();
@@ -1755,13 +1735,12 @@ int sumcheck_run(qz_ctx* ctx, size_t num_vars, size_t k, const void* const* tabl
       gather_par = (int)(ctx->gather_seq++ & 1);
     }
     {
-      const void* kern = nullptr;
+      auto kern = sc_mid<0>;
       switch (cp.product_k) {
-        case 1: kern = (const void*)sc_mid<1>; break;
-        case 2: kern = (const void*)sc_mid<2>; break;
-        case 3: kern = (const void*)sc_mid<3>; break;
-        case 4: kern = (const void*)sc_mid<4>; break;
-        default: kern = (const void*)sc_mid<0>;
+        case 1: kern = sc_mid<1>; break;
+        case 2: kern = sc_mid<2>; break;
+        case 3: kern = sc_mid<3>; break;
+        case 4: kern = sc_mid<4>; break;
       }
       // the grid: as many blocks as the widest remaining round uses (the kernel derives every round's share from
       // gridDim.x with the same plan), all co-resident, and never more than a block has threads (the closing block
@@ -1771,33 +1750,25 @@ int sumcheck_run(qz_ctx* ctx, size_t num_vars, size_t k, const void* const* tabl
       const unsigned int cap = (unsigned int)std::min<uint64_t>(SC_THREADS, (uint64_t)ctx->sm_count * occ);
       ScMidPlan plan;
       const int grid = (int)mid_make_plan(plan, size, pending, ka, d, cap, mid_G);
-      ScTables k_tabs = tabs;
-      uint64_t k_size = size;
-      int k_pending = pending, k_round = round, k_mc = mc, k_rank = ctx->rank, k_G = mid_G, k_zc_n = zerocheck ? (int)num_vars : 0;
-      ScHead* k_head = head;
-      const ScProgram* k_prog = d_prog;
-      const Fr *k_consts = d_consts, *k_vinv = vinv, *k_z = d_z;
-      Fr *k_coeffs = d_coeffs, *k_point = d_point, *k_parts = partials;
-      uint32_t* k_lens = d_lens;
-      PeerMailbox* const* k_peers = (PeerMailbox* const*)ctx->peer_mbox_dev;
-      void* args[] = {&k_tabs, &tb, &k_size, &k_pending, &k_head, &k_prog, &k_consts, &k_vinv, &k_coeffs, &k_lens, &k_point,
-                      &k_round, &k_mc, &k_parts, &d_sync, &k_peers, &k_rank, &k_G, &seq0, &gather_par, &k_z, &k_zc_n, &plan};
+      cudaLaunchConfig_t cfg = {};
+      cfg.gridDim = dim3(grid);
+      cfg.blockDim = dim3(SC_THREADS);
+      cfg.stream = st;
+      cudaLaunchAttribute at[1];
       if (grid > 1) {  // the blocks wait for one another: they must all be resident
-        QZ_CUDA(ctx, cudaLaunchCooperativeKernel(kern, dim3(grid), dim3(SC_THREADS), args, 0, st));
-        ctx->launches++;
+        at[0].id = cudaLaunchAttributeCooperative;
+        at[0].val.cooperative = 1;
       } else {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(1);
-        cfg.blockDim = dim3(SC_THREADS);
-        cfg.stream = st;
-        cudaLaunchAttribute at[1];
         at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         at[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = at;
-        cfg.numAttrs = (pdl_ok && G == 1) ? 1 : 0;
-        QZ_CUDA(ctx, cudaLaunchKernelExC(&cfg, kern, args));
-        ctx->launches++;
       }
+      cfg.attrs = at;
+      cfg.numAttrs = grid > 1 || (pdl_ok && G == 1) ? 1 : 0;
+      QZ_CUDA(ctx, cudaLaunchKernelEx(&cfg, kern, tabs, tb, size, pending, head, (const ScProgram*)d_prog,
+                                      (const Fr*)d_consts, (const Fr*)vinv, d_coeffs, d_lens, d_point, round, mc, partials,
+                                      d_sync, (PeerMailbox* const*)ctx->peer_mbox_dev, ctx->rank, mid_G, seq0, gather_par,
+                                      (const Fr*)d_z, zerocheck ? (int)num_vars : 0, plan));
+      ctx->launches++;
     }
   }
 
@@ -1808,13 +1779,10 @@ int sumcheck_run(qz_ctx* ctx, size_t num_vars, size_t k, const void* const* tabl
   const ScHead* h = (const ScHead*)(pin_out + o_head);
   if (h->peer_fault == 2) return ctx->fail(QZ_ERR_CUDA, "a block of the persistent round kernel never saw its round closed");
   if (h->peer_fault) return ctx->fail(QZ_ERR_NCCL, "a peer did not deliver its partial sums (peer mailbox wait timed out)");
-  if (zc_skip1 && h->zc_degenerate) {  // some z_j = 0 (probability 2^-254 per challenge): redo without the 1 / z_j shortcut
-    tl_zc_no_skip = true;              // every rank draws the same z, so every rank takes this branch
-    rc = sumcheck_run(ctx, num_vars, k, tables, tables_on_device, nodes, n_nodes, consts, n_consts, claimed_sum, state,
-                      max_coeffs, out_coeffs, out_lens, out_point, out_eval, zerocheck, out_z, sharded);
-    tl_zc_no_skip = false;
-    return rc;
-  }
+  if (zc_skip1 && h->zc_degenerate)  // some z_j = 0 (probability 2^-254 per challenge): redo without the 1 / z_j shortcut
+    return sumcheck_prove(ctx, num_vars, k, tables, tables_on_device, nodes, n_nodes, consts, n_consts, claimed_sum,
+                          state, max_coeffs, out_coeffs, out_lens, out_point, out_eval, zerocheck, out_z, sharded,
+                          false);  // every rank draws the same z, so every rank takes this branch
   memcpy(state, h->tstate, 32);
   memcpy(out_eval, h->evaluation.v, 32);
   if (num_vars) {
@@ -1827,6 +1795,15 @@ int sumcheck_run(qz_ctx* ctx, size_t num_vars, size_t k, const void* const* tabl
   if (num_vars > 0) cudaEventElapsedTime(&ctx->last_ms[1], ctx->ev_k0, ctx->ev_k1);
   else ctx->last_ms[1] = 0.f;
   return QZ_OK;
+}
+
+int sumcheck_run(qz_ctx* ctx, size_t num_vars, size_t k, const void* const* tables, int tables_on_device,
+                 const qz_expr_node* nodes, size_t n_nodes, const uint8_t* consts, size_t n_consts,
+                 const uint8_t* claimed_sum, uint8_t* state, size_t max_coeffs, uint8_t* out_coeffs,
+                 uint32_t* out_lens, uint8_t* out_point, uint8_t* out_eval, bool zerocheck, uint8_t* out_z,
+                 bool sharded) {
+  return sumcheck_prove(ctx, num_vars, k, tables, tables_on_device, nodes, n_nodes, consts, n_consts, claimed_sum, state,
+                        max_coeffs, out_coeffs, out_lens, out_point, out_eval, zerocheck, out_z, sharded, true);
 }
 
 }  // namespace qz
