@@ -224,8 +224,10 @@ __global__ void __launch_bounds__(32) msm_sum_points_peers(const uint8_t* mine_x
     affine_store(out_affine, xyzz_to_affine_serial(total));
   }
 }
+}  // extern "C"
+
 // all ranks' partial sums (`mine`: 128 B XYZZ on the device) -> affine sum on every rank
-static int msm_exchange_sum(qz_ctx* ctx, uint8_t* mine, uint8_t* all, uint8_t* out_dev) {
+int qz::msm_exchange_sum(qz_ctx* ctx, uint8_t* mine, uint8_t* all, uint8_t* out_dev, uint32_t** pinned_fault) {
   const int G = ctx->nranks > 0 ? ctx->nranks : 1;
   if (G > 1 && qz::comm_has_peers(ctx)) {
     uint32_t* fault = (uint32_t*)ctx->arena_alloc(4);
@@ -236,7 +238,7 @@ static int msm_exchange_sum(qz_ctx* ctx, uint8_t* mine, uint8_t* all, uint8_t* o
     uint32_t* pin = (uint32_t*)ctx->pinned_buf(64);
     if (!pin) return ctx->fail(QZ_ERR_ALLOC, "pinned");
     QZ_CUDA(ctx, cudaMemcpyAsync(pin, fault, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    ctx->pending_fault = pin;
+    *pinned_fault = pin;
     return QZ_OK;
   }
   if (G > 1) {
@@ -248,84 +250,18 @@ static int msm_exchange_sum(qz_ctx* ctx, uint8_t* mine, uint8_t* all, uint8_t* o
   return qz::msm_sum_points_launch(ctx, all, G, out_dev);
 }
 
+extern "C" {
+
 int qz_msm_sharded(qz_ctx* ctx, const qz_srs* srs, const void* scalars, size_t n_scalars, int on_device,
                    uint8_t out_xy[64]) {
-  if (!ctx || !srs || !out_xy || (n_scalars && !scalars)) return QZ_ERR_INVALID_ARG;
-  QZ_CUDA(ctx, cudaSetDevice(ctx->device));
-  ctx->arena_reset();
-  const size_t n = std::min(n_scalars, srs->n);
-  cudaStream_t st = ctx->stream;
-  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_call0, st));
-  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_k0, st));
-  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_k1, st));
-  uint4* sdev = (uint4*)scalars;
-  const void* shost = nullptr;
-  if (!on_device && n) {
-    sdev = (uint4*)ctx->arena_alloc(32 * n);
-    if (!sdev) return ctx->fail(QZ_ERR_ALLOC, "scalars");
-    shost = scalars;
-  }
-  uint8_t* mine = (uint8_t*)ctx->arena_alloc(128);
-  uint8_t* all = (uint8_t*)ctx->arena_alloc((size_t)128 * ctx->nranks);
-  uint8_t* out_dev = (uint8_t*)ctx->arena_alloc(64);
-  if (!mine || !all || !out_dev) return ctx->fail(QZ_ERR_ALLOC, "result");
-  int rc = msm_run(ctx, srs, sdev, shost, n, mine, nullptr);
-  if (rc) return rc;
-  rc = msm_exchange_sum(ctx, mine, all, out_dev);
-  if (rc) return rc;
-  QZ_CUDA(ctx, cudaMemcpyAsync(out_xy, out_dev, 64, cudaMemcpyDeviceToHost, st));
-  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_call1, st));
-  QZ_CUDA(ctx, cudaStreamSynchronize(st));
-  if (ctx->pending_fault && *ctx->pending_fault) {
-    ctx->pending_fault = nullptr;
-    return ctx->fail(QZ_ERR_NCCL, "a peer did not deliver its partial sum (peer mailbox wait timed out)");
-  }
-  ctx->pending_fault = nullptr;
-  cudaEventElapsedTime(&ctx->last_ms[0], ctx->ev_call0, ctx->ev_call1);
-  ctx->last_ms[1] = msm_accumulate_ms(ctx);
-  return QZ_OK;
+  return msm_call(ctx, srs, scalars, n_scalars, on_device, MsmMode::sharded, out_xy);
 }
 
 // The same product when every rank holds the WHOLE SRS and the WHOLE scalar vector (HyperPlonk's witness and logup
 // commits at N > 1): rank g takes the index range [n g / G, n (g + 1) / G), the 128-byte partial sums are gathered
 // and added on every rank.  Without a communicator it is qz_kzg_commit.
 int qz_msm_split(qz_ctx* ctx, const qz_srs* srs, const void* scalars, size_t n_scalars, int on_device, uint8_t out_xy[64]) {
-  if (!ctx || !srs || !out_xy || (n_scalars && !scalars)) return QZ_ERR_INVALID_ARG;
-  if (n_scalars > srs->n) return ctx->fail(QZ_ERR_DEGREE, "Polynomial degree exceeds max degree");
-  QZ_CUDA(ctx, cudaSetDevice(ctx->device));
-  ctx->arena_reset();
-  const int G = ctx->nranks > 0 ? ctx->nranks : 1;
-  const size_t lo = n_scalars * (size_t)ctx->rank / G, hi = n_scalars * ((size_t)ctx->rank + 1) / G, n = hi - lo;
-  cudaStream_t st = ctx->stream;
-  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_call0, st));
-  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_k0, st));
-  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_k1, st));
-  uint4* sdev = on_device ? (uint4*)scalars + 2 * lo : nullptr;
-  const void* shost = nullptr;
-  if (!on_device && n) {
-    sdev = (uint4*)ctx->arena_alloc(32 * n);
-    if (!sdev) return ctx->fail(QZ_ERR_ALLOC, "scalars");
-    shost = (const uint8_t*)scalars + 32 * lo;
-  }
-  uint8_t* mine = (uint8_t*)ctx->arena_alloc(128);
-  uint8_t* all = (uint8_t*)ctx->arena_alloc((size_t)128 * G);
-  uint8_t* out_dev = (uint8_t*)ctx->arena_alloc(64);
-  if (!mine || !all || !out_dev) return ctx->fail(QZ_ERR_ALLOC, "result");
-  int rc = msm_run(ctx, srs, sdev, shost, n, mine, nullptr, lo);
-  if (rc) return rc;
-  rc = msm_exchange_sum(ctx, mine, all, out_dev);
-  if (rc) return rc;
-  QZ_CUDA(ctx, cudaMemcpyAsync(out_xy, out_dev, 64, cudaMemcpyDeviceToHost, st));
-  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_call1, st));
-  QZ_CUDA(ctx, cudaStreamSynchronize(st));
-  if (ctx->pending_fault && *ctx->pending_fault) {
-    ctx->pending_fault = nullptr;
-    return ctx->fail(QZ_ERR_NCCL, "a peer did not deliver its partial sum (peer mailbox wait timed out)");
-  }
-  ctx->pending_fault = nullptr;
-  cudaEventElapsedTime(&ctx->last_ms[0], ctx->ev_call0, ctx->ev_call1);
-  ctx->last_ms[1] = msm_accumulate_ms(ctx);
-  return QZ_OK;
+  return msm_call(ctx, srs, scalars, n_scalars, on_device, MsmMode::split, out_xy);
 }
 
 // Re-agree on the mailbox sequence numbers after a sharded call failed somewhere (a rank that left a call early -- an

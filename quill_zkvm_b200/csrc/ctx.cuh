@@ -149,7 +149,6 @@ struct qz_ctx {
   void** peer_mbox_dev = nullptr;
   void* peer_mbox_host[16] = {};
   uint32_t mbox_seq = 0;
-  uint32_t* pending_fault = nullptr;  // pinned word the current sharded MSM's exchange kernel reports a peer timeout in
   uint32_t gather_seq = 0;  // sharded sumchecks handed over through the mailboxes' gather areas so far (picks the copy)
 
   int fail(int status, const char* what, cudaError_t ce = cudaSuccess) {

@@ -3,26 +3,26 @@
 // Reference: KZG::commit (pcs/src/kzg.rs:61-73), whose work is ark-ec 0.5.0's VariableBaseMSM::msm_unchecked on the
 // affine-normalised SRS; KZG::open (pcs/src/kzg.rs:75-96); KZG::trusted_setup's G1 powers (pcs/src/kzg.rs:35-59).
 //
-// Pipeline (all on the device, one stream):
-//   1. msm_digits        scalar: Montgomery -> canonical -> signed c-bit digits; one (key, value) per (window, scalar)
+// Pipeline (msm_run, after msm_plan; the first three stages run per range of the points, see segment_weights):
+//   prep_segment         on the prep stream when there are several ranges, overlapped with the previous accumulation:
+//     msm_digits         scalar: Montgomery -> canonical -> signed c-bit digits; one (key, value) per (window, scalar)
 //                        key = window << c | |digit|, value = point index | sign << 31
-//   2. radix sort        (key, value) pairs by key (cub::DeviceRadixSort) -> every bucket's points are contiguous
-//   3. msm_accumulate    the hot kernel: the sorted list is cut into fixed chunks of 32..128 entries, one thread per
+//     radix sort         (key, value) pairs by key (cub::DeviceRadixSort) -> every bucket's points are contiguous
+//   pair_levels          optional (QZ_MSM_PAIR_LEVELS = k, off by default): k halvings of the sorted list by affine
+//                        additions with a shared inversion (msm_pair_*, section 4b below; DESIGN.md section 3)
+//   msm_accumulate       the hot kernel: the sorted list is cut into fixed chunks of 32..128 entries, one thread per
 //                        chunk, XYZZ += affine (8M + 2S) per entry with the next base prefetched; load is balanced
 //                        whatever the scalar distribution.  A chunk's first / last runs may be partial buckets and go
 //                        to a list of partial runs, interior runs are complete buckets and are written in place.
-//  3b. msm_pair_*        optional (QZ_MSM_PAIR_LEVELS = k, off by default): k halvings of the sorted list by affine
-//                        additions with a shared inversion before step 3 (section 4b below; DESIGN.md section 3)
-//   4. msm_partials_reduce  the list of partial runs is reduced by the same chunked rule, level by level, until it
-//                        fits one chunk: no thread ever walks a whole bucket, however skewed the scalars are
-//   5. msm_bucket_reduce per window: sum_b b * B_b by segmented running sums + a tree reduction
-//   6. msm_combine       Horner over windows (c doublings each) + one inversion to affine
+//   reduce_partial_runs  the list of partial runs is reduced by the same chunked rule, level by level, until it fits
+//                        one chunk: no thread ever walks a whole bucket, however skewed the scalars are
+//   reduce_and_combine   the ranges' bucket copies are added; per window sum_b b * B_b by segmented running sums + a
+//                        tree reduction; Horner over windows (c doublings each) + one inversion to affine
 // Bases are normalised to affine ONCE at SRS upload; the reference re-normalises on every commit (kzg.rs:67-71).
 #include <cub/cub.cuh>
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
-#include <memory>
 #include <new>
 #include "ctx.cuh"
 #include "ec.cuh"
@@ -874,11 +874,266 @@ static int segment_weights(bool host_scalars, size_t n, double* w) {
   return 1;
 }
 
-// sum_i scalars[i] * srs->bases[i], i < n.  The scalars are Montgomery Fr, either already on the device (scalars_host
-// null) or in host memory, in which case `scalars_dev` is the device buffer they are copied into, range by range.
-// Writes the result as XYZZ (128 B, device) and/or affine (64 B, device).  `srs` supplies the bases and, when present
-// and cheaper by the cost model, the precomputed window multiples.  Asynchronous: everything is ordered on ctx->stream
-// when the call returns (the prep stream is joined before the last accumulation).
+// Every choice of one MSM, made on the host before anything is allocated or enqueued.
+struct MsmPlan {
+  int c, Wd, W;             // window bits, digits per scalar, bucket sets (1 when collapsed)
+  bool collapsed;           // all windows share one bucket set through the precomputed multiples srs->pre
+  const uint8_t* bases;     // srs->pre when collapsed, else srs->bases
+  uint64_t m;               // sorted entries: Wd per scalar
+  int key_bits;             // bits the sort orders by: (segment, window, digit)
+  uint32_t per_w, n_slots;  // buckets per set, buckets of one segment's W sets
+  int pair_levels;
+  int chunk_len;            // sorted entries per accumulate thread
+  int S;                    // point ranges [seg_lo[s], seg_lo[s + 1]), each with its own copy of the bucket sets
+  size_t seg_lo[qz_ctx::MAX_SEGMENTS + 1], max_seg;
+  uint64_t chunk_base[qz_ctx::MAX_SEGMENTS + 1];  // range s accumulates chunks [chunk_base[s], chunk_base[s + 1])
+  int seg;                  // buckets per bucket-reduce thread
+  uint32_t red_threads, per_window_parts;
+  // partial-run lists: level 0 has two slots per accumulate chunk, level k+1 two per PART_CHUNK slots of level k
+  uint64_t n_part0, n_part1;
+};
+
+static int msm_plan(qz_ctx* ctx, const qz_srs* srs, size_t n, bool host_scalars, MsmPlan& p) {
+  if (n >= ((size_t)1 << 31)) return ctx->fail(QZ_ERR_INVALID_ARG, "MSM size must be below 2^31");
+  p.c = pick_window(n);
+  p.collapsed = srs->pre && msm_cost(n, srs->pre_c, true) < msm_cost(n, p.c, false);
+  if (p.collapsed) p.c = srs->pre_c;
+  const int c = p.c;
+  p.Wd = (256 + c - 1) / c;
+  p.W = p.collapsed ? 1 : p.Wd;
+  p.bases = p.collapsed ? srs->pre : srs->bases;
+  p.m = (uint64_t)p.Wd * n;
+  ctx->last_stat[0] = c;
+  ctx->last_stat[1] = p.Wd;
+  ctx->last_stat[2] = p.collapsed ? 1 : 0;
+  ctx->last_stat[3] = (double)p.m;
+  if (p.m >= ((uint64_t)1 << 32)) return ctx->fail(QZ_ERR_INVALID_ARG, "MSM too large for 32-bit positions");
+  p.per_w = 1u << (c - 1);
+  p.n_slots = (uint32_t)p.W * p.per_w;
+  p.key_bits = c;
+  while ((1u << (p.key_bits - c)) < (uint32_t)p.W) p.key_bits++;
+  // pair levels ahead of the accumulation (QZ_MSM_PAIR_LEVELS = count; unset: none): values need bit 30 as the flag
+  p.pair_levels = 0;
+  const char* env = getenv("QZ_MSM_PAIR_LEVELS");
+  if (env && *env) p.pair_levels = std::max(0, std::min(PAIR_MAX_LEVELS, atoi(env)));
+  const uint64_t max_index = (p.collapsed ? (uint64_t)p.Wd * srs->n : (uint64_t)srs->n);
+  if (p.m >= VAL_PAIR || max_index >= VAL_PAIR || p.m < 64) p.pair_levels = 0;
+  // chunk length: at least ~16 chunks per resident accumulate thread, else the minimum.  The pair levels leave the
+  // accumulation a list ~2^levels shorter: the chunks are sized for that list, so that enough of them fill the machine.
+  p.chunk_len = (int)std::min<uint64_t>(ACC_CHUNK_MAX, (p.m >> p.pair_levels) / ((uint64_t)ctx->sm_count * 4 * ACC_THREADS * 16));
+  p.chunk_len = std::max(ACC_CHUNK_MIN, p.chunk_len / 32 * 32);
+
+  double weights[qz_ctx::MAX_SEGMENTS];
+  const int S = segment_weights(host_scalars, n, weights);
+  double total = 0, run = 0;
+  for (int s = 0; s < S; s++) total += weights[s];
+  p.S = 0;
+  p.seg_lo[0] = 0;
+  for (int s = 0; s < S; s++) {
+    run += weights[s];
+    size_t hi = s == S - 1 ? n : std::min(n, ((size_t)((double)n * run / total) + 255) & ~(size_t)255);
+    if (hi > p.seg_lo[p.S]) p.seg_lo[++p.S] = hi;
+  }
+  if (((uint64_t)p.S * p.W) << c >= 0xffffffffull) {  // (segment, window, digit) must fit the 32-bit key below KEY_NONE
+    p.S = 1;
+    p.seg_lo[1] = n;
+  }
+  p.chunk_base[0] = 0;
+  p.max_seg = 0;
+  for (int s = 0; s < p.S; s++) {
+    const uint64_t ms = (uint64_t)p.Wd * (p.seg_lo[s + 1] - p.seg_lo[s]);
+    p.chunk_base[s + 1] = p.chunk_base[s] + (ms + p.chunk_len - 1) / p.chunk_len;
+    p.max_seg = std::max(p.max_seg, p.seg_lo[s + 1] - p.seg_lo[s]);
+  }
+  p.n_part0 = 2 * p.chunk_base[p.S];
+  p.n_part1 = 2 * ((p.n_part0 + PART_CHUNK - 1) / PART_CHUNK);
+  // small problems are latency-bound: shorter running-sum segments (more threads, shorter dependent chains)
+  // large bucket sets: one wave of threads (2^15 x 64 buckets at c = 22) beats two waves of shorter chains
+  // (2^19 buckets, one rank's share of 2^24 points on 8 GPUs: 16K threads walking 32 buckets are latency-bound, 0.63 ms)
+  const uint32_t n_slots = p.n_slots;
+  const int seg_want = n_slots <= (1u << 17) ? 8 : n_slots <= (1u << 19) ? RED_SEG / 2 : n_slots >= (1u << 21) ? 2 * RED_SEG : RED_SEG;
+  p.seg = p.per_w >= (uint32_t)seg_want ? seg_want : (int)p.per_w;
+  p.red_threads = n_slots / p.seg;
+  p.per_window_parts = p.per_w / p.seg;
+  return QZ_OK;
+}
+
+// pair levels (msm_pair_*): scratch for the longest range, shared by the ranges (they run in turn on the main stream)
+struct PairScratch {
+  PairCtl* ctl;
+  uint8_t *sums, *prefix, *codes;
+  uint8_t *v[PAIR_TREE_MAX + 1], *pre[PAIR_TREE_MAX];  // inversion tree: elements / running products per depth
+  unsigned long long *counts, *offs;
+  void* scan_tmp;
+  size_t scan_bytes;
+};
+struct MsmScratch {
+  uint32_t *keys, *vals, *keys2, *vals2;  // the (key, value) list and the sort's second buffer
+  uint8_t* buckets;                        // S copies of the bucket sets
+  uint8_t *ppts_a, *ppts_b;                // partial-run lists (n_part0 / n_part1 slots) and their keys
+  uint32_t *pkeys_a, *pkeys_b;
+  uint8_t *fin_a, *fin_b;                  // msm_partials_finish's scan buffers
+  uint8_t *partial, *partial2, *window_sums;
+  void* sort_tmp;  // shared: the segments' sorts are serialised on the prep stream
+  size_t sort_bytes;
+  PairScratch pairs;                       // allocated only with pair levels
+};
+
+static int msm_scratch(qz_ctx* ctx, const MsmPlan& p, cudaStream_t ps, MsmScratch& sc) {
+  bool ok = true;
+  auto take = [&](size_t bytes) {
+    void* q = ctx->arena_alloc(bytes);
+    ok = ok && q;
+    return q;
+  };
+  sc.keys = (uint32_t*)take(4 * p.m);
+  sc.vals = (uint32_t*)take(4 * p.m);
+  sc.keys2 = (uint32_t*)take(4 * p.m);
+  sc.vals2 = (uint32_t*)take(4 * p.m);
+  sc.buckets = (uint8_t*)take((size_t)p.S * p.n_slots * 128);
+  sc.ppts_a = (uint8_t*)take(p.n_part0 * 128);
+  sc.pkeys_a = (uint32_t*)take(p.n_part0 * 4);
+  sc.ppts_b = (uint8_t*)take(p.n_part1 * 128);
+  sc.pkeys_b = (uint32_t*)take(p.n_part1 * 4);
+  sc.fin_a = (uint8_t*)take((size_t)FIN_SLOTS * 128);
+  sc.fin_b = (uint8_t*)take((size_t)FIN_SLOTS * 128);
+  sc.partial = (uint8_t*)take((size_t)p.red_threads * 128);
+  sc.partial2 = (uint8_t*)take((size_t)p.W * ((p.per_window_parts + SUM_SPAN - 1) / SUM_SPAN) * 128);
+  sc.window_sums = (uint8_t*)take((size_t)p.W * 128);
+  cub::DoubleBuffer<uint32_t> dk(sc.keys, sc.keys2), dv(sc.vals, sc.vals2);
+  cub::DeviceRadixSort::SortPairs(nullptr, sc.sort_bytes, dk, dv, (int64_t)((uint64_t)p.Wd * p.max_seg), 0, p.key_bits, ps);
+  sc.sort_tmp = take(sc.sort_bytes);
+  if (!ok) return ctx->fail(QZ_ERR_ALLOC, "MSM scratch");
+  if (!p.pair_levels) return QZ_OK;
+
+  PairScratch& pr = sc.pairs;
+  const uint64_t mmax = (uint64_t)p.Wd * p.max_seg;
+  const uint64_t tiles = (mmax + 2 * PAIR_TILE - 1) / (2 * PAIR_TILE);
+  pr.ctl = (PairCtl*)take(sizeof(PairCtl));
+  pr.sums = (uint8_t*)take(mmax * 64);
+  pr.prefix = (uint8_t*)take(tiles * PAIR_TILE * 32);
+  pr.codes = (uint8_t*)take(tiles * PAIR_TILE);
+  uint64_t n = tiles * PAIR_THREADS;
+  for (int k = 0; k <= PAIR_TREE_MAX; k++) {
+    pr.v[k] = (uint8_t*)take(n * 32);
+    if (n == 1) break;
+    if (k == PAIR_TREE_MAX) {
+      ok = false;
+      break;
+    }
+    pr.pre[k] = (uint8_t*)take(n * 32);
+    n = (n + PAIR_G - 1) / PAIR_G;
+  }
+  pr.counts = (unsigned long long*)take((tiles + 1) * 8);
+  pr.offs = (unsigned long long*)take((tiles + 1) * 8);
+  cub::DeviceScan::ExclusiveSum(nullptr, pr.scan_bytes, pr.counts, pr.offs, (int64_t)(tiles + 1), ctx->stream);
+  pr.scan_tmp = take(pr.scan_bytes);
+  if (!ok) return ctx->fail(QZ_ERR_ALLOC, "MSM pair-level scratch");
+  return QZ_OK;
+}
+
+// On return dk / dv hold range s's sorted list in Current() and the sort's other buffer in Alternate().
+static int prep_segment(qz_ctx* ctx, const qz_srs* srs, const MsmPlan& p, MsmScratch& sc, int s, cudaStream_t ps,
+                        uint4* scalars_dev, const void* scalars_host, size_t first, cub::DoubleBuffer<uint32_t>& dk,
+                        cub::DoubleBuffer<uint32_t>& dv) {
+  QzRange nvtx("qz:msm:digits+sort");
+  const size_t lo = p.seg_lo[s], ns = p.seg_lo[s + 1] - lo;
+  const uint64_t off = (uint64_t)p.Wd * lo;
+  if (scalars_host)
+    QZ_CUDA(ctx, cudaMemcpyAsync(scalars_dev + 2 * lo, (const uint8_t*)scalars_host + 32 * lo, 32 * ns,
+                                 cudaMemcpyHostToDevice, ps));
+  QZ_LAUNCH_ON(ctx, ps, msm_digits, (unsigned)((ns + 255) / 256), 256, 0, scalars_dev + 2 * lo, (uint32_t)ns,
+               (uint32_t)(first + lo), p.c, p.Wd, p.collapsed ? (uint32_t)srs->n : 0u, (uint32_t)(s * p.W), sc.keys + off,
+               sc.vals + off, ctx->acc_ring_on ? ctx->acc_nonzero_dev : nullptr);
+  dk = cub::DoubleBuffer<uint32_t>(sc.keys + off, sc.keys2 + off);
+  dv = cub::DoubleBuffer<uint32_t>(sc.vals + off, sc.vals2 + off);
+  QZ_CUDA(ctx, cub::DeviceRadixSort::SortPairs(sc.sort_tmp, sc.sort_bytes, dk, dv, (int64_t)((uint64_t)p.Wd * ns), 0,
+                                               p.key_bits, ps));
+  ctx->launches += 2 + (p.key_bits + 7) / 8;  // CUB: histogram + one onesweep pass per 8 key bits (approximate)
+  if (p.S > 1) {
+    QZ_CUDA(ctx, cudaEventRecord(ctx->ev_seg_ready[s], ps));
+    QZ_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_seg_ready[s], 0));
+  }
+  return QZ_OK;
+}
+
+// Each level reads dk / dv's Current() buffers and writes their Alternate() ones, which then become Current().
+static int pair_levels(qz_ctx* ctx, const MsmPlan& p, PairScratch& pr, uint64_t ms, cub::DoubleBuffer<uint32_t>& dk,
+                       cub::DoubleBuffer<uint32_t>& dv) {
+  const uint64_t tiles = (ms + 2 * PAIR_TILE - 1) / (2 * PAIR_TILE);  // of a level over the longest list possible
+  uint64_t tree_n[PAIR_TREE_MAX + 1];  // elements per depth over the longest list possible, down to ONE root
+  int tree_depth = 0;
+  tree_n[0] = tiles * PAIR_THREADS;
+  while (tree_n[tree_depth] > 1) {
+    tree_n[tree_depth + 1] = (tree_n[tree_depth] + PAIR_G - 1) / PAIR_G;
+    tree_depth++;
+  }
+  const uint32_t dmask = (1u << p.c) - 1;
+  QZ_LAUNCH(ctx, msm_pair_init, 1, 1, 0, pr.ctl, ms, pr.counts + tiles);
+  for (int l = 0; l < p.pair_levels; l++) {
+    QZ_LAUNCH(ctx, msm_pair_scan, (unsigned)tiles, PAIR_THREADS, 0, dk.Current(), dv.Current(), pr.ctl, l, dmask, p.bases,
+              pr.sums, pr.prefix, pr.v[0], pr.codes, pr.counts);
+    QZ_CUDA(ctx, cub::DeviceScan::ExclusiveSum(pr.scan_tmp, pr.scan_bytes, pr.counts, pr.offs, (int64_t)(tiles + 1),
+                                               ctx->stream));
+    ctx->launches += 2;
+    for (int k = 0; k < tree_depth; k++)
+      QZ_LAUNCH(ctx, msm_pair_tree_up, (unsigned)((tree_n[k + 1] + 127) / 128), 128, 0, pr.ctl, l, k, pr.v[k], pr.pre[k],
+                pr.v[k + 1]);
+    QZ_LAUNCH(ctx, msm_pair_tree_root, 1, 1, 0, pr.ctl, l, pr.v[tree_depth]);
+    for (int k = tree_depth - 1; k >= 0; k--)
+      QZ_LAUNCH(ctx, msm_pair_tree_down, (unsigned)((tree_n[k + 1] + 127) / 128), 128, 0, pr.ctl, l, k, pr.v[k], pr.pre[k],
+                pr.v[k + 1]);
+    QZ_LAUNCH(ctx, msm_pair_apply, (unsigned)tiles, PAIR_THREADS, 0, dk.Current(), dv.Current(), pr.ctl, l, dmask, p.bases,
+              pr.sums, pr.prefix, pr.v[0], pr.codes, pr.offs, (uint32_t)tiles, dk.Alternate(), dv.Alternate());
+    dk.selector ^= 1;
+    dv.selector ^= 1;
+  }
+  return QZ_OK;
+}
+
+// Merge the partial runs level by level until one chunk holds them all (one list: the segments' keys ascend).
+static int reduce_partial_runs(qz_ctx* ctx, const MsmPlan& p, const MsmScratch& sc) {
+  QzRange nvtx("qz:msm:partial-runs");
+  uint32_t *kin = sc.pkeys_a, *kout = sc.pkeys_b;
+  uint8_t *pin = sc.ppts_a, *pout = sc.ppts_b;
+  uint64_t n_in = p.n_part0;
+  while (true) {
+    if (n_in <= (uint64_t)FIN_SLOTS && n_in > PART_CHUNK) {  // short list: scan it in one launch
+      QZ_LAUNCH(ctx, msm_partials_finish, 1, FIN_THREADS, 0, kin, pin, (int)n_in, p.c, sc.buckets, sc.fin_a, sc.fin_b);
+      return QZ_OK;
+    }
+    const uint64_t chunks = (n_in + PART_CHUNK - 1) / PART_CHUNK;
+    const int last_level = chunks == 1;
+    QZ_LAUNCH(ctx, msm_partials_reduce, (unsigned)((chunks + 127) / 128), 128, 0, kin, pin, n_in, p.c, sc.buckets, kout, pout,
+              last_level);
+    if (last_level) return QZ_OK;
+    n_in = 2 * chunks;
+    // the output of this level (<= n_part1 slots) becomes the input; the other buffer is large enough
+    std::swap(kin, kout);
+    std::swap(pin, pout);
+  }
+}
+
+static int reduce_and_combine(qz_ctx* ctx, const MsmPlan& p, const MsmScratch& sc, uint8_t* out_xyzz_dev,
+                              uint8_t* out_affine_dev) {
+  QzRange nvtx("qz:msm:bucket-reduce+combine");
+  if (p.S > 1) QZ_LAUNCH(ctx, msm_bucket_merge, (p.n_slots + 127) / 128, 128, 0, sc.buckets, p.n_slots, p.S);
+  QZ_LAUNCH(ctx, msm_bucket_reduce, (p.red_threads + 127) / 128, 128, 0, sc.buckets, p.c, p.W, p.seg, sc.partial);
+  uint8_t *in = sc.partial, *out = sc.partial2;  // per window: per_window_parts partial sums -> 1
+  uint32_t per_in = p.per_window_parts;
+  while (per_in > SUM_SPAN) {
+    const uint32_t per_out = (per_in + SUM_SPAN - 1) / SUM_SPAN;
+    QZ_LAUNCH(ctx, msm_block_sum, (unsigned)p.W * per_out, 128, 0, in, per_in, per_out, out);
+    std::swap(in, out);
+    per_in = per_out;
+  }
+  QZ_LAUNCH(ctx, msm_block_sum, (unsigned)p.W, 128, 0, in, per_in, 1u, sc.window_sums);
+  QZ_LAUNCH(ctx, msm_combine, 1, 1, 0, sc.window_sums, p.c, p.W, out_xyzz_dev, out_affine_dev);
+  return QZ_OK;
+}
+
+// `srs` supplies the bases and, when present and cheaper by the cost model, the precomputed window multiples.  Everything
+// is ordered on ctx->stream when the call returns (the prep stream is joined before the last accumulation).
 int msm_run(qz_ctx* ctx, const qz_srs* srs, uint4* scalars_dev, const void* scalars_host, size_t n,
             uint8_t* out_xyzz_dev, uint8_t* out_affine_dev, size_t first) {
   cudaStream_t st = ctx->stream;
@@ -889,261 +1144,49 @@ int msm_run(qz_ctx* ctx, const qz_srs* srs, uint4* scalars_dev, const void* scal
     if (out_affine_dev) QZ_CUDA(ctx, cudaMemsetAsync(out_affine_dev, 0, 64, st));
     return QZ_OK;
   }
-  if (n >= ((size_t)1 << 31)) return ctx->fail(QZ_ERR_INVALID_ARG, "MSM size must be below 2^31");
+  MsmPlan p;
+  int rc = msm_plan(ctx, srs, n, scalars_host != nullptr, p);
+  if (rc) return rc;
+  if (p.S > 1 && ctx->ensure_prep_stream()) return ctx->fail(QZ_ERR_CUDA, "prep stream");
+  cudaStream_t ps = p.S > 1 ? ctx->prep_stream : st;
   auto mark = ctx->arena_mark();
-  int c = pick_window(n);
-  const bool collapsed = srs->pre && msm_cost(n, srs->pre_c, true) < msm_cost(n, c, false);
-  if (collapsed) c = srs->pre_c;
-  const int Wd = (256 + c - 1) / c;       // digits per scalar
-  const int W = collapsed ? 1 : Wd;       // bucket sets
-  const uint8_t* bases = collapsed ? srs->pre : srs->bases;
-  const uint64_t m = (uint64_t)Wd * n;
-  ctx->last_stat[0] = c;
-  ctx->last_stat[1] = Wd;
-  ctx->last_stat[2] = collapsed ? 1 : 0;
-  ctx->last_stat[3] = (double)m;
-  if (m >= ((uint64_t)1 << 32)) return ctx->fail(QZ_ERR_INVALID_ARG, "MSM too large for 32-bit positions");
-  const uint32_t per_w = 1u << (c - 1), n_slots = (uint32_t)W * per_w;
-  // chunk length: at least ~16 chunks per resident accumulate thread, else the minimum
-  int chunk_len = (int)std::min<uint64_t>(ACC_CHUNK_MAX, m / ((uint64_t)ctx->sm_count * 4 * ACC_THREADS * 16));
-  chunk_len = std::max(ACC_CHUNK_MIN, chunk_len / 32 * 32);
-  int key_bits = c;
-  while ((1u << (key_bits - c)) < (uint32_t)W) key_bits++;
-  // pair levels ahead of the accumulation (QZ_MSM_PAIR_LEVELS = count; unset: none): values need bit 30 as the flag
-  int pair_levels = 0;
-  {
-    const char* env = getenv("QZ_MSM_PAIR_LEVELS");
-    if (env && *env) pair_levels = std::max(0, std::min(PAIR_MAX_LEVELS, atoi(env)));
-    const uint64_t max_index = (collapsed ? (uint64_t)Wd * srs->n : (uint64_t)srs->n);
-    if (m >= VAL_PAIR || max_index >= VAL_PAIR || m < 64) pair_levels = 0;
-  }
-  if (pair_levels) {  // the list the accumulation sees is ~2^levels shorter: keep enough chunks to fill the machine
-    chunk_len = (int)std::min<uint64_t>(ACC_CHUNK_MAX, (m >> pair_levels) / ((uint64_t)ctx->sm_count * 4 * ACC_THREADS * 16));
-    chunk_len = std::max(ACC_CHUNK_MIN, chunk_len / 32 * 32);
-  }
+  MsmScratch sc{};
+  rc = msm_scratch(ctx, p, ps, sc);
+  if (rc) return rc;
 
-  // point ranges [seg_lo[s], seg_lo[s+1])
-  double weights[qz_ctx::MAX_SEGMENTS];
-  int S = segment_weights(scalars_host != nullptr, n, weights);
-  size_t seg_lo[qz_ctx::MAX_SEGMENTS + 1];
-  {
-    double total = 0, run = 0;
-    for (int s = 0; s < S; s++) total += weights[s];
-    int kept = 0;
-    seg_lo[0] = 0;
-    for (int s = 0; s < S; s++) {
-      run += weights[s];
-      size_t hi = s == S - 1 ? n : std::min(n, ((size_t)((double)n * run / total) + 255) & ~(size_t)255);
-      if (hi > seg_lo[kept]) seg_lo[++kept] = hi;
-    }
-    S = kept;
-  }
-  if (((uint64_t)S * W) << c >= 0xffffffffull) {  // (segment, window, digit) must fit the 32-bit key below KEY_NONE
-    S = 1;
-    seg_lo[1] = n;
-  }
-  if (S > 1 && ctx->ensure_prep_stream()) return ctx->fail(QZ_ERR_CUDA, "prep stream");
-  cudaStream_t ps = S > 1 ? ctx->prep_stream : st;
-  uint64_t chunk_base[qz_ctx::MAX_SEGMENTS + 1];
-  chunk_base[0] = 0;
-  size_t max_seg = 0;
-  for (int s = 0; s < S; s++) {
-    const uint64_t ms = (uint64_t)Wd * (seg_lo[s + 1] - seg_lo[s]);
-    chunk_base[s + 1] = chunk_base[s] + (ms + chunk_len - 1) / chunk_len;
-    max_seg = std::max(max_seg, seg_lo[s + 1] - seg_lo[s]);
-  }
-  const uint64_t n_chunks = chunk_base[S];
-
-  uint32_t* keys = (uint32_t*)ctx->arena_alloc(4 * m);
-  uint32_t* vals = (uint32_t*)ctx->arena_alloc(4 * m);
-  uint32_t* keys2 = (uint32_t*)ctx->arena_alloc(4 * m);
-  uint32_t* vals2 = (uint32_t*)ctx->arena_alloc(4 * m);
-  uint8_t* buckets = (uint8_t*)ctx->arena_alloc((size_t)S * n_slots * 128);
-  // partial-run lists: level 0 has two slots per accumulate chunk, level k+1 two per PART_CHUNK slots of level k
-  const uint64_t n_part0 = 2 * n_chunks, n_part1 = 2 * ((n_part0 + PART_CHUNK - 1) / PART_CHUNK);
-  uint8_t* ppts_a = (uint8_t*)ctx->arena_alloc(n_part0 * 128);
-  uint32_t* pkeys_a = (uint32_t*)ctx->arena_alloc(n_part0 * 4);
-  uint8_t* ppts_b = (uint8_t*)ctx->arena_alloc(n_part1 * 128);
-  uint32_t* pkeys_b = (uint32_t*)ctx->arena_alloc(n_part1 * 4);
-  uint8_t* fin_a = (uint8_t*)ctx->arena_alloc((size_t)FIN_SLOTS * 128);
-  uint8_t* fin_b = (uint8_t*)ctx->arena_alloc((size_t)FIN_SLOTS * 128);
-  // small problems are latency-bound: shorter running-sum segments (more threads, shorter dependent chains)
-  // large bucket sets: one wave of threads (2^15 x 64 buckets at c = 22) beats two waves of shorter chains
-  // (2^19 buckets, one rank's share of 2^24 points on 8 GPUs: 16K threads walking 32 buckets are latency-bound, 0.63 ms)
-  const int seg_want = n_slots <= (1u << 17) ? 8 : n_slots <= (1u << 19) ? RED_SEG / 2 : n_slots >= (1u << 21) ? 2 * RED_SEG : RED_SEG;
-  const int seg = per_w >= (uint32_t)seg_want ? seg_want : (int)per_w;
-  const uint32_t red_threads = n_slots / seg, per_window_parts = per_w / seg;
-  uint8_t* partial = (uint8_t*)ctx->arena_alloc((size_t)red_threads * 128);
-  uint8_t* partial2 = (uint8_t*)ctx->arena_alloc((size_t)W * ((per_window_parts + SUM_SPAN - 1) / SUM_SPAN) * 128);
-  uint8_t* window_sums = (uint8_t*)ctx->arena_alloc((size_t)W * 128);
-  size_t sort_bytes = 0;
-  {
-    cub::DoubleBuffer<uint32_t> dk(keys, keys2), dv(vals, vals2);
-    cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, dk, dv, (int64_t)((uint64_t)Wd * max_seg), 0, key_bits, ps);
-  }
-  void* sort_tmp = ctx->arena_alloc(sort_bytes);  // shared: the segments' sorts are serialised on the prep stream
-  if (!keys || !vals || !keys2 || !vals2 || !buckets || !ppts_a || !pkeys_a || !ppts_b || !pkeys_b || !fin_a || !fin_b || !partial ||
-      !partial2 || !window_sums || !sort_tmp)
-    return ctx->fail(QZ_ERR_ALLOC, "MSM scratch");
-  // pair levels (msm_pair_*): scratch for the longest segment, shared by the segments (they run in turn on `st`)
-  PairCtl* pair_ctl = nullptr;
-  uint8_t *pair_sums = nullptr, *pair_prefix = nullptr, *pair_codes = nullptr;
-  uint8_t *pair_v[PAIR_TREE_MAX + 1] = {}, *pair_pre[PAIR_TREE_MAX] = {};  // inversion tree: elements / running products per depth
-  unsigned long long *pair_counts = nullptr, *pair_offs = nullptr;
-  void* pair_scan_tmp = nullptr;
-  size_t pair_scan_bytes = 0;
-  if (pair_levels) {
-    const uint64_t mmax = (uint64_t)Wd * max_seg;
-    const uint64_t tiles = (mmax + 2 * PAIR_TILE - 1) / (2 * PAIR_TILE);
-    pair_ctl = (PairCtl*)ctx->arena_alloc(sizeof(PairCtl));
-    pair_sums = (uint8_t*)ctx->arena_alloc(mmax * 64);
-    pair_prefix = (uint8_t*)ctx->arena_alloc(tiles * PAIR_TILE * 32);
-    pair_codes = (uint8_t*)ctx->arena_alloc(tiles * PAIR_TILE);
-    bool tree_ok = true;
-    {
-      uint64_t n = tiles * PAIR_THREADS;
-      for (int k = 0; k <= PAIR_TREE_MAX; k++) {
-        pair_v[k] = (uint8_t*)ctx->arena_alloc(n * 32);
-        tree_ok = tree_ok && pair_v[k];
-        if (n == 1) break;
-        if (k == PAIR_TREE_MAX) {
-          tree_ok = false;
-          break;
-        }
-        pair_pre[k] = (uint8_t*)ctx->arena_alloc(n * 32);
-        tree_ok = tree_ok && pair_pre[k];
-        n = (n + PAIR_G - 1) / PAIR_G;
-      }
-    }
-    pair_counts = (unsigned long long*)ctx->arena_alloc((tiles + 1) * 8);
-    pair_offs = (unsigned long long*)ctx->arena_alloc((tiles + 1) * 8);
-    cub::DeviceScan::ExclusiveSum(nullptr, pair_scan_bytes, pair_counts, pair_offs, (int64_t)(tiles + 1), st);
-    pair_scan_tmp = ctx->arena_alloc(pair_scan_bytes);
-    if (!pair_ctl || !pair_sums || !pair_prefix || !pair_codes || !tree_ok || !pair_counts || !pair_offs || !pair_scan_tmp)
-      return ctx->fail(QZ_ERR_ALLOC, "MSM pair-level scratch");
-  }
-
-  if (S > 1) {  // the prep stream starts where the main stream stands (earlier users of the scratch, the scalars)
+  if (p.S > 1) {  // the prep stream starts where the main stream stands (earlier users of the scratch, the scalars)
     QZ_CUDA(ctx, cudaEventRecord(ctx->ev_entry, st));
     QZ_CUDA(ctx, cudaStreamWaitEvent(ps, ctx->ev_entry, 0));
   }
-  QZ_CUDA(ctx, cudaMemsetAsync(buckets, 0, (size_t)S * n_slots * 128, st));
-  for (int s = 0; s < S; s++) {
-    const size_t lo = seg_lo[s], ns = seg_lo[s + 1] - lo;
-    const uint64_t off = (uint64_t)Wd * lo, ms = (uint64_t)Wd * ns;
-    std::unique_ptr<QzRange> nvtx_prep(new QzRange("qz:msm:digits+sort"));
-    if (scalars_host)
-      QZ_CUDA(ctx, cudaMemcpyAsync(scalars_dev + 2 * lo, (const uint8_t*)scalars_host + 32 * lo, 32 * ns,
-                                   cudaMemcpyHostToDevice, ps));
-    QZ_LAUNCH_ON(ctx, ps, msm_digits, (unsigned)((ns + 255) / 256), 256, 0, scalars_dev + 2 * lo, (uint32_t)ns,
-                 (uint32_t)(first + lo), c, Wd, collapsed ? (uint32_t)srs->n : 0u, (uint32_t)(s * W), keys + off, vals + off,
-                 ctx->acc_ring_on ? ctx->acc_nonzero_dev : nullptr);
-    cub::DoubleBuffer<uint32_t> dk(keys + off, keys2 + off), dv(vals + off, vals2 + off);
-    QZ_CUDA(ctx, cub::DeviceRadixSort::SortPairs(sort_tmp, sort_bytes, dk, dv, (int64_t)ms, 0, key_bits, ps));
-    ctx->launches += 2 + (key_bits + 7) / 8;  // CUB: histogram + one onesweep pass per 8 key bits (approximate)
-    if (S > 1) {
-      QZ_CUDA(ctx, cudaEventRecord(ctx->ev_seg_ready[s], ps));
-      QZ_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev_seg_ready[s], 0));
-    }
-    nvtx_prep.reset();
+  QZ_CUDA(ctx, cudaMemsetAsync(sc.buckets, 0, (size_t)p.S * p.n_slots * 128, st));
+  const auto accumulate = p.pair_levels ? msm_accumulate<true> : msm_accumulate<false>;
+  for (int s = 0; s < p.S; s++) {
+    cub::DoubleBuffer<uint32_t> dk, dv;
+    rc = prep_segment(ctx, srs, p, sc, s, ps, scalars_dev, scalars_host, first, dk, dv);
+    if (rc) return rc;
     QzRange nvtx_acc("qz:msm:accumulate");
+    const uint64_t ms = (uint64_t)p.Wd * (p.seg_lo[s + 1] - p.seg_lo[s]), chunks = p.chunk_base[s + 1] - p.chunk_base[s];
     cudaEvent_t ring0 = nullptr, ring1 = nullptr;
     const bool ring = ctx->acc_ring_next(&ring0, &ring1) == 0;
     if (ring) QZ_CUDA(ctx, cudaEventRecord(ring0, st));
-    QZ_CUDA(ctx, cudaEventRecord(S > 1 ? ctx->ev_acc0[s] : ctx->ev_k0, st));
-    const uint64_t seg_chunks = chunk_base[s + 1] - chunk_base[s];
-    if (pair_levels) {
-      uint32_t* kbuf[2] = {dk.Current(), dk.Alternate()};  // a level reads one buffer of the sort's pair and writes the other
-      uint32_t* vbuf[2] = {dv.Current(), dv.Alternate()};
-      int cur = 0;
-      const uint64_t tiles = (ms + 2 * PAIR_TILE - 1) / (2 * PAIR_TILE);  // of a level over the longest list possible
-      uint64_t tree_n[PAIR_TREE_MAX + 1];  // elements per depth over the longest list possible, down to ONE root
-      int tree_depth = 0;
-      tree_n[0] = tiles * PAIR_THREADS;
-      while (tree_n[tree_depth] > 1) {
-        tree_n[tree_depth + 1] = (tree_n[tree_depth] + PAIR_G - 1) / PAIR_G;
-        tree_depth++;
-      }
-      const uint32_t dmask = (1u << c) - 1;
-      QZ_LAUNCH(ctx, msm_pair_init, 1, 1, 0, pair_ctl, ms, pair_counts + tiles);
-      for (int l = 0; l < pair_levels; l++) {
-        const uint32_t* kc = kbuf[cur];
-        const uint32_t* vc = vbuf[cur];
-        QZ_LAUNCH(ctx, msm_pair_scan, (unsigned)tiles, PAIR_THREADS, 0, kc, vc, pair_ctl, l, dmask, bases, pair_sums, pair_prefix,
-                  pair_v[0], pair_codes, pair_counts);
-        QZ_CUDA(ctx, cub::DeviceScan::ExclusiveSum(pair_scan_tmp, pair_scan_bytes, pair_counts, pair_offs, (int64_t)(tiles + 1), st));
-        ctx->launches += 2;
-        for (int k = 0; k < tree_depth; k++)
-          QZ_LAUNCH(ctx, msm_pair_tree_up, (unsigned)((tree_n[k + 1] + 127) / 128), 128, 0, pair_ctl, l, k, pair_v[k], pair_pre[k],
-                    pair_v[k + 1]);
-        QZ_LAUNCH(ctx, msm_pair_tree_root, 1, 1, 0, pair_ctl, l, pair_v[tree_depth]);
-        for (int k = tree_depth - 1; k >= 0; k--)
-          QZ_LAUNCH(ctx, msm_pair_tree_down, (unsigned)((tree_n[k + 1] + 127) / 128), 128, 0, pair_ctl, l, k, pair_v[k], pair_pre[k],
-                    pair_v[k + 1]);
-        QZ_LAUNCH(ctx, msm_pair_apply, (unsigned)tiles, PAIR_THREADS, 0, kc, vc, pair_ctl, l, dmask, bases, pair_sums, pair_prefix,
-                  pair_v[0], pair_codes, pair_offs, (uint32_t)tiles, kbuf[cur ^ 1], vbuf[cur ^ 1]);
-        cur ^= 1;
-      }
-      QZ_LAUNCH(ctx, msm_accumulate<true>, (unsigned)((seg_chunks + ACC_THREADS - 1) / ACC_THREADS), ACC_THREADS, 0,
-                (const uint32_t*)kbuf[cur], (const uint32_t*)vbuf[cur], (uint64_t)0, &pair_ctl->m[pair_levels], seg_chunks, chunk_len, bases, pair_sums, c, buckets,
-                ppts_a + chunk_base[s] * 256, pkeys_a + 2 * chunk_base[s]);
-    } else {
-      QZ_LAUNCH(ctx, msm_accumulate<false>, (unsigned)((seg_chunks + ACC_THREADS - 1) / ACC_THREADS), ACC_THREADS, 0,
-                dk.Current(), dv.Current(), ms, (const uint64_t*)nullptr, seg_chunks, chunk_len, bases,
-                (const uint8_t*)nullptr, c, buckets, ppts_a + chunk_base[s] * 256, pkeys_a + 2 * chunk_base[s]);
-    }
-    QZ_CUDA(ctx, cudaEventRecord(S > 1 ? ctx->ev_acc1[s] : ctx->ev_k1, st));
+    QZ_CUDA(ctx, cudaEventRecord(p.S > 1 ? ctx->ev_acc0[s] : ctx->ev_k0, st));
+    rc = p.pair_levels ? pair_levels(ctx, p, sc.pairs, ms, dk, dv) : QZ_OK;
+    if (rc) return rc;
+    QZ_LAUNCH(ctx, accumulate, (unsigned)((chunks + ACC_THREADS - 1) / ACC_THREADS), ACC_THREADS, 0, dk.Current(),
+              dv.Current(), p.pair_levels ? 0 : ms, p.pair_levels ? &sc.pairs.ctl->m[p.pair_levels] : nullptr, chunks,
+              p.chunk_len, p.bases, sc.pairs.sums, p.c, sc.buckets, sc.ppts_a + p.chunk_base[s] * 256,
+              sc.pkeys_a + 2 * p.chunk_base[s]);
+    QZ_CUDA(ctx, cudaEventRecord(p.S > 1 ? ctx->ev_acc1[s] : ctx->ev_k1, st));
     if (ring) {
       QZ_CUDA(ctx, cudaEventRecord(ring1, st));
       ctx->acc_ring_adds += (double)ms;  // sorted entries; the additions executed are counted by msm_digits
     }
   }
-  ctx->acc_launches = S > 1 ? S : 0;
-  {  // merge partial runs level by level until one chunk holds them all (one list: the segments' keys ascend)
-    QzRange nvtx_parts("qz:msm:partial-runs");
-    const uint32_t* kin = pkeys_a;
-    const uint8_t* pin = ppts_a;
-    uint32_t* kout = pkeys_b;
-    uint8_t* pout = ppts_b;
-    uint64_t n_in = n_part0;
-    while (true) {
-      if (n_in <= (uint64_t)FIN_SLOTS && n_in > PART_CHUNK) {  // short list: scan it in one launch
-        QZ_LAUNCH(ctx, msm_partials_finish, 1, FIN_THREADS, 0, kin, pin, (int)n_in, c, buckets, fin_a, fin_b);
-        break;
-      }
-      const uint64_t chunks = (n_in + PART_CHUNK - 1) / PART_CHUNK;
-      const int last_level = chunks == 1;
-      QZ_LAUNCH(ctx, msm_partials_reduce, (unsigned)((chunks + 127) / 128), 128, 0, kin, pin, n_in, c, buckets, kout, pout,
-                last_level);
-      if (last_level) break;
-      n_in = 2 * chunks;
-      // ping-pong: the output of this level (<= n_part1 slots) becomes the input; the other buffer is large enough
-      const uint32_t* tk = kin;
-      const uint8_t* tp = pin;
-      kin = kout;
-      pin = pout;
-      kout = const_cast<uint32_t*>(tk);
-      pout = const_cast<uint8_t*>(tp);
-    }
-  }
-  QzRange nvtx_red("qz:msm:bucket-reduce+combine");
-  if (S > 1) QZ_LAUNCH(ctx, msm_bucket_merge, (n_slots + 127) / 128, 128, 0, buckets, n_slots, S);
-  QZ_LAUNCH(ctx, msm_bucket_reduce, (red_threads + 127) / 128, 128, 0, buckets, c, W, seg, partial);
-  {  // per window: per_window_parts partial sums -> 1
-    const uint8_t* in = partial;
-    uint32_t per_in = per_window_parts;
-    uint8_t* bufs[2] = {partial2, partial};
-    int flip = 0;
-    while (per_in > SUM_SPAN) {
-      const uint32_t per_out = (per_in + SUM_SPAN - 1) / SUM_SPAN;
-      QZ_LAUNCH(ctx, msm_block_sum, (unsigned)W * per_out, 128, 0, in, per_in, per_out, bufs[flip]);
-      in = bufs[flip];
-      per_in = per_out;
-      flip ^= 1;
-    }
-    QZ_LAUNCH(ctx, msm_block_sum, (unsigned)W, 128, 0, in, per_in, 1u, window_sums);
-  }
-  QZ_LAUNCH(ctx, msm_combine, 1, 1, 0, window_sums, c, W, out_xyzz_dev, out_affine_dev);
+  ctx->acc_launches = p.S > 1 ? p.S : 0;
+  rc = reduce_partial_runs(ctx, p, sc);
+  if (rc) return rc;
+  rc = reduce_and_combine(ctx, p, sc, out_xyzz_dev, out_affine_dev);
+  if (rc) return rc;
   ctx->arena_release(mark);  // stream order keeps the scratch valid for the kernels enqueued above
   return QZ_OK;
 }
@@ -1151,21 +1194,6 @@ int msm_run(qz_ctx* ctx, const qz_srs* srs, uint4* scalars_dev, const void* scal
 int msm_device(qz_ctx* ctx, const qz_srs* srs, const uint4* scalars_dev, size_t n, uint8_t* out_xyzz_dev,
                uint8_t* out_affine_dev) {
   return msm_run(ctx, srs, const_cast<uint4*>(scalars_dev), nullptr, n, out_xyzz_dev, out_affine_dev);
-}
-
-// duration of the last MSM's accumulate launches (call after the stream is synchronised)
-float msm_accumulate_ms(qz_ctx* ctx) {
-  float total = 0.f;
-  if (ctx->acc_launches == 0) {
-    cudaEventElapsedTime(&total, ctx->ev_k0, ctx->ev_k1);
-    return total;
-  }
-  for (int s = 0; s < ctx->acc_launches; s++) {
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, ctx->ev_acc0[s], ctx->ev_acc1[s]);
-    total += ms;
-  }
-  return total;
 }
 
 // KZG::open (kzg.rs:75-96) with everything on the device: x is read from device memory, y (32 B) and the affine proof
@@ -1207,6 +1235,54 @@ int kzg_open_device(qz_ctx* ctx, const qz_srs* srs, const uint4* pdev, size_t n_
 
 int msm_sum_points_launch(qz_ctx* ctx, const uint8_t* pts_dev, int n, uint8_t* out_affine_dev) {
   QZ_LAUNCH(ctx, msm_sum_points, 1, 1, 0, pts_dev, n, out_affine_dev);
+  return QZ_OK;
+}
+
+int msm_call(qz_ctx* ctx, const qz_srs* srs, const void* scalars, size_t n_scalars, int on_device, MsmMode mode,
+             uint8_t out_xy[64]) {
+  if (!ctx || !srs || !out_xy || (n_scalars && !scalars)) return QZ_ERR_INVALID_ARG;
+  if (mode == MsmMode::split && n_scalars > srs->n) return ctx->fail(QZ_ERR_DEGREE, "Polynomial degree exceeds max degree");
+  QZ_CUDA(ctx, cudaSetDevice(ctx->device));
+  ctx->arena_reset();
+  const int G = ctx->nranks > 0 ? ctx->nranks : 1;
+  size_t lo = 0, n = std::min(n_scalars, srs->n);  // msm_unchecked zips to the shorter slice
+  if (mode == MsmMode::split) {
+    lo = n_scalars * (size_t)ctx->rank / G;
+    n = n_scalars * ((size_t)ctx->rank + 1) / G - lo;
+  }
+  cudaStream_t st = ctx->stream;
+  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_call0, st));
+  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_k0, st));
+  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_k1, st));
+  uint4* sdev = on_device ? (uint4*)scalars + 2 * lo : nullptr;
+  const void* shost = nullptr;
+  if (!on_device && n) {  // the copy is issued range by range inside msm_run, overlapped with the accumulation
+    sdev = (uint4*)ctx->arena_alloc(32 * n);
+    if (!sdev) return ctx->fail(QZ_ERR_ALLOC, "scalars");
+    shost = (const uint8_t*)scalars + 32 * lo;
+  }
+  const bool exchange = mode != MsmMode::local;  // this rank's XYZZ partial sum `mine`, added to the other ranks' ones
+  uint8_t* mine = exchange ? (uint8_t*)ctx->arena_alloc(128) : nullptr;
+  uint8_t* all = exchange ? (uint8_t*)ctx->arena_alloc((size_t)128 * G) : nullptr;
+  uint8_t* out_dev = (uint8_t*)ctx->arena_alloc(64);
+  if ((exchange && (!mine || !all)) || !out_dev) return ctx->fail(QZ_ERR_ALLOC, "result");
+  int rc = msm_run(ctx, srs, sdev, shost, n, mine, exchange ? nullptr : out_dev, lo);
+  uint32_t* fault = nullptr;
+  if (!rc && exchange) rc = msm_exchange_sum(ctx, mine, all, out_dev, &fault);
+  if (rc) return rc;
+  QZ_CUDA(ctx, cudaMemcpyAsync(out_xy, out_dev, 64, cudaMemcpyDeviceToHost, st));
+  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_call1, st));
+  QZ_CUDA(ctx, cudaStreamSynchronize(st));
+  if (fault && *fault) return ctx->fail(QZ_ERR_NCCL, "a peer did not deliver its partial sum (peer mailbox wait timed out)");
+  cudaEventElapsedTime(&ctx->last_ms[0], ctx->ev_call0, ctx->ev_call1);
+  float acc = 0.f;  // the msm_accumulate launches: between ev_k0 and ev_k1, or one event pair per range
+  if (ctx->acc_launches == 0) cudaEventElapsedTime(&acc, ctx->ev_k0, ctx->ev_k1);
+  for (int s = 0; s < ctx->acc_launches; s++) {
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, ctx->ev_acc0[s], ctx->ev_acc1[s]);
+    acc += ms;
+  }
+  ctx->last_ms[1] = acc;
   return QZ_OK;
 }
 
@@ -1312,31 +1388,7 @@ int qz_srs_download(qz_ctx* ctx, const qz_srs* s, size_t first, size_t count, ui
 }
 
 int qz_msm(qz_ctx* ctx, const qz_srs* srs, const void* scalars, size_t n_scalars, int on_device, uint8_t out_xy[64]) {
-  if (!ctx || !srs || !out_xy || (n_scalars && !scalars)) return QZ_ERR_INVALID_ARG;
-  QZ_CUDA(ctx, cudaSetDevice(ctx->device));
-  ctx->arena_reset();
-  const size_t n = std::min(n_scalars, srs->n);  // msm_unchecked zips to the shorter slice
-  cudaStream_t st = ctx->stream;
-  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_call0, st));
-  uint4* sdev = (uint4*)scalars;
-  const void* shost = nullptr;
-  if (!on_device && n) {  // the copy is issued range by range inside msm_run, overlapped with the accumulation
-    sdev = (uint4*)ctx->arena_alloc(32 * n);
-    if (!sdev) return ctx->fail(QZ_ERR_ALLOC, "scalars");
-    shost = scalars;
-  }
-  uint8_t* out_dev = (uint8_t*)ctx->arena_alloc(64);
-  if (!out_dev) return ctx->fail(QZ_ERR_ALLOC, "result");
-  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_k0, st));
-  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_k1, st));
-  int rc = msm_run(ctx, srs, sdev, shost, n, nullptr, out_dev);
-  if (rc) return rc;
-  QZ_CUDA(ctx, cudaMemcpyAsync(out_xy, out_dev, 64, cudaMemcpyDeviceToHost, st));
-  QZ_CUDA(ctx, cudaEventRecord(ctx->ev_call1, st));
-  QZ_CUDA(ctx, cudaStreamSynchronize(st));
-  cudaEventElapsedTime(&ctx->last_ms[0], ctx->ev_call0, ctx->ev_call1);
-  ctx->last_ms[1] = msm_accumulate_ms(ctx);
-  return QZ_OK;
+  return msm_call(ctx, srs, scalars, n_scalars, on_device, MsmMode::local, out_xy);
 }
 
 int qz_kzg_commit(qz_ctx* ctx, const qz_srs* srs, const void* coeffs, size_t n_coeffs, int on_device,

@@ -23,11 +23,18 @@ int msm_device(qz_ctx* ctx, const qz_srs* srs, const uint4* scalars_dev, size_t 
 // first, first + 1, .. (a rank's index range of an MSM over an SRS every rank holds: qz_msm_split)
 int msm_run(qz_ctx* ctx, const qz_srs* srs, uint4* scalars_dev, const void* scalars_host, size_t n,
             uint8_t* out_xyzz_dev, uint8_t* out_affine_dev, size_t first = 0);
-// duration of the last MSM's msm_accumulate launches, summed (valid once ctx->stream is synchronised)
-float msm_accumulate_ms(qz_ctx* ctx);
 // KZG::open on the device: x read from device memory, y (32 B) and the affine proof (64 B) written to device memory
 int kzg_open_device(qz_ctx* ctx, const qz_srs* srs, const uint4* pdev, size_t n_coeffs,
                     const Fp<FrParams>* x_dev, Fp<FrParams>* y_dev, uint8_t* proof_affine_dev);
 // affine(sum of n XYZZ points on the device) -> out_affine_dev (64 B)
 int msm_sum_points_launch(qz_ctx* ctx, const uint8_t* pts_dev, int n, uint8_t* out_affine_dev);
+// every rank's XYZZ partial sum `mine` (128 B, device; `all`: 128 B per rank) -> their affine sum in out_dev.  With peer
+// mailboxes *pinned_fault is set to a pinned word that is non-zero after the stream synchronises if a peer timed out.
+int msm_exchange_sum(qz_ctx* ctx, uint8_t* mine, uint8_t* all, uint8_t* out_dev, uint32_t** pinned_fault);
+
+// the C-ABI MSMs qz_msm, qz_msm_sharded and qz_msm_split, by `mode`: arguments checked, scalars staged, the affine
+// result copied to out_xy (host memory) and the call's timings recorded
+enum class MsmMode { local, sharded, split };
+int msm_call(qz_ctx* ctx, const qz_srs* srs, const void* scalars, size_t n_scalars, int on_device, MsmMode mode,
+             uint8_t out_xy[64]);
 }  // namespace qz

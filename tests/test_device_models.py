@@ -8,7 +8,7 @@ is pinned independently of the GPU tests:
   * blake3 compression with the state columns spread over four lanes (csrc/sumcheck.cuh b3_compress_quad)
   * the inverse by the binary extended Euclidean algorithm (csrc/ff.cuh fp_inv_serial)
   * the merge of partial bucket runs by a segmented scan with early exit (csrc/msm.cu msm_partials_finish)
-  * the streamed MSM's point ranges (csrc/msm.cu msm_run)
+  * the streamed MSM's point ranges (csrc/msm.cu msm_plan)
   * NTT passes as plain local transforms + one correction product per element (csrc/mlpcs.cu ntt_pass)
   * the K = 3 round polynomial from samples at X = 0, 1, -1, infinity with lazily added operands, X = 1 restored from the
     running claim (csrc/sumcheck.cu prod_core_toom3, csrc/sumcheck.cuh sc_expand_evals / sc_toom3_to_coeffs)
@@ -248,7 +248,7 @@ def test_segmented_scan_merges_partial_runs():
 
 # ---------------------------------------------------------------------------------------------------------------------
 def segment_bounds(n, weights):
-    """msm_run: cumulative weights -> range ends rounded up to 256 points, empty ranges dropped, last end = n"""
+    """msm_plan: cumulative weights -> range ends rounded up to 256 points, empty ranges dropped, last end = n"""
     total, run, lo = sum(weights), 0.0, [0]
     for s, w in enumerate(weights):
         run += w
